@@ -4,7 +4,7 @@
 A "step" is one pass of the hot path over one batch of 1024 synthetic depth-32 withdraw witnesses:
 MiMC7 Merkle-path witness generation -> A.w/B.w -> 6 NTTs -> 3 fixed-base MSMs -> 256-byte proofs.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 `value`   : whole-job proofs/s with the secret inputs already resident in HBM (og_*_dev entry points),
             timed with CUDA events on the library's stream, max over ranks.
@@ -18,6 +18,10 @@ MiMC7 Merkle-path witness generation -> A.w/B.w -> 6 NTTs -> 3 fixed-base MSMs -
             reference arm.
 Multi-GPU: proofs are independent -> one process per GPU, each proving its own batch (weak scaling),
 no data-path collective; NCCL is used only for the barrier and the max-over-ranks reduction.
+
+--dump-outputs DIR: after the timed steps, the proofs and public inputs of the last timed step (rank 0) go to
+DIR/proofs.npy and DIR/public_inputs.npy, one row per proof, byte values as float32.  The inputs are seeded, so two
+builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -37,6 +41,8 @@ BATCH = 1024
 METRIC = "groth16_withdraw_proofs_per_sec"
 UNIT = "proofs/s"
 TOXIC_SEED = 20260922
+INPUT_SEED = 4096               # + rank: the secret inputs of the timed batch
+DUMP_BYTES = 64 << 20           # cap on what --dump-outputs writes
 
 
 def measured_peaks():
@@ -118,6 +124,20 @@ def parse_pk_blob(pk: bytes, n_vars, n_pub, log_m):
         out[name] = pk[o:o + size]; o += size
     out["log_m"] = log_m
     return out
+
+
+def dump_outputs(out_dir, proofs: bytes, pub: bytes, n: int):
+    """--dump-outputs: n proofs (256 B) and their public inputs (96 B) as float32 arrays of byte values (exact);
+    a batch too large for DUMP_BYTES is written as a fixed, seeded sample of rows."""
+    import numpy as np
+    rows = np.arange(n)
+    cap = DUMP_BYTES // (4 * (256 + 96))
+    if n > cap:
+        rows = np.sort(np.random.default_rng(0).choice(n, cap, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, b, w in (("proofs", proofs, 256), ("public_inputs", pub, 96)):
+        a = np.frombuffer(b, dtype=np.uint8).reshape(n, w)[rows].astype(np.float32)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def physical_cores():
@@ -310,8 +330,11 @@ def run_reference(args):
         pr.prove_batch(wit, rs)
     t = time.perf_counter()
     for _ in range(args.steps):
-        pr.prove_batch(wit, rs)
+        proofs = pr.prove_batch(wit, rs)
     dt = time.perf_counter() - t
+    if args.dump_outputs:
+        nv = cs.n_vars
+        dump_outputs(args.dump_outputs, proofs, b"".join(wit[32 * nv * i + 32:32 * nv * i + 128] for i in range(sample)), sample)
     value = sample * args.steps / dt
     one = cpu_single_thread_seconds(pr, random.Random(11))
     line = {
@@ -342,7 +365,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true", help=argparse.SUPPRESS)
     ap.add_argument("--no-parity", action="store_true", help=argparse.SUPPRESS)
     ap.add_argument("--sharded-log-n", type=int, default=22, help=argparse.SUPPRESS)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's proofs and public inputs to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -366,7 +392,7 @@ def main():
     rng = random.Random(TOXIC_SEED)
     pk_bytes, vk_bytes = ob.setup_withdraw(ctx, DEPTH, *toxic(rng))
     PK = ob.ProvingKey(ctx, pk_bytes)
-    nul, sec, rec, sib, bits, rs = synth_inputs(random.Random(4096 + rank), batch, DEPTH)
+    nul, sec, rec, sib, bits, rs = synth_inputs(random.Random(INPUT_SEED + rank), batch, DEPTH)
 
     def dev_u8(b):
         return torch.frombuffer(bytearray(b), dtype=torch.uint8).to(dev)
@@ -413,6 +439,8 @@ def main():
     # below (rank 0), four of them are compared byte for byte with the oracle's C prover
     proofs_host = bytes(d_proofs.cpu().numpy().tobytes())
     pub_host = bytes(d_pub.cpu().numpy().tobytes())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, proofs_host, pub_host, batch)
     vidx = sorted({(i * batch) // 16 for i in range(16)} | {batch - 1})
     n_verified = sum(bool(ob.verify(vk_bytes, pub_host[96 * i:96 * i + 96], proofs_host[256 * i:256 * i + 256])) for i in vidx)
     verified = n_verified == len(vidx)
@@ -446,7 +474,7 @@ def main():
     sharded = None
     if args.sharded_log_n > 0:
         try:
-            sharded = sharded_msm_leg(torch, dist, ob, api, ctx, dev, rank, world, args.sharded_log_n)
+            sharded = sharded_msm_leg(torch, dist, ob, api, ctx, dev, rank, world, args.sharded_log_n, steps=args.steps)
         except Exception as e:      # an extra leg: its failure must not hide the headline
             sharded = {"error": f"{type(e).__name__}: {e}"}
 

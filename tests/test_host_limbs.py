@@ -16,8 +16,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 @pytest.fixture(scope="module")
-def h():
-    so = os.path.join(ROOT, "tests", "harness", "libhost_harness.so")
+def h(tmp_path_factory):
+    so = str(tmp_path_factory.mktemp("harness") / "libhost_harness.so")
     src = os.path.join(ROOT, "tests", "harness", "host_harness.cpp")
     subprocess.run(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-I" + os.path.join(ROOT, "owshen_b200", "csrc"),
                     "-o", so, src], check=True)
