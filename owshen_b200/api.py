@@ -11,7 +11,7 @@ import os
 import subprocess
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# OWSHEN_B200_LIB: an alternative build of the same library (A/B experiments of compile-time variants)
+# OWSHEN_B200_LIB: an alternative build of the same library (e.g. another commit's, for an A/B)
 _LIB_PATH = os.environ.get("OWSHEN_B200_LIB") or os.path.join(_HERE, "libowshen_b200.so")
 _lib = None
 

@@ -2,7 +2,6 @@
 // Host-pointer entry points stage their buffers in persistent device slots (H2D/D2H on the ctx
 // stream, truly asynchronous when the caller's memory is pinned) and return after the result has
 // landed; `_dev` entry points only enqueue.  No entry point has a CPU implementation.
-#include <stdlib.h>
 #include "common.cuh"
 #include "groth16.cuh"
 #include "mimc.cuh"
@@ -15,7 +14,7 @@ using namespace og;
 void* og_ctx::slot(int id, size_t bytes) {
     if (bytes == 0) bytes = 32;
     if (slot_cap[id] >= bytes) return slot_ptr[id];
-    cudaDeviceSynchronize();          // growth is rare; other lanes may still be using neighbouring slots' kernels
+    cudaDeviceSynchronize();          // growth is rare; work already enqueued may still be using the old buffer
     if (slot_ptr[id]) cudaFree(slot_ptr[id]);
     slot_ptr[id] = nullptr; slot_cap[id] = 0;
     size_t cap = bytes + bytes / 8;
@@ -107,19 +106,6 @@ int32_t og_init(int32_t device, og_ctx** out) {
         return OG_E_CUDA;
     }
     cudaMemset(ctx->d_flag, 0, sizeof(int));
-    ctx->main_stream = ctx->stream;
-    {
-        int least = 0, greatest = 0;
-        cudaDeviceGetStreamPriorityRange(&least, &greatest);
-        { const char* v = getenv("OG_LANE_PRIO"); if (v && atoi(v) == 0) least = greatest = 0; }   // A/B: lanes without stream priorities
-        bool ok = cudaEventCreateWithFlags(&ctx->fork_ev, cudaEventDisableTiming) == cudaSuccess &&
-                  cudaEventCreateWithFlags(&ctx->acc_ev, cudaEventDisableTiming) == cudaSuccess;
-        for (int l = 0; ok && l < MAX_LANES; l++)
-            ok = cudaStreamCreateWithPriority(&ctx->lane_hi[l], cudaStreamNonBlocking, greatest) == cudaSuccess &&
-                 cudaStreamCreateWithPriority(&ctx->lane_lo[l], cudaStreamNonBlocking, least) == cudaSuccess &&
-                 cudaEventCreateWithFlags(&ctx->lane_ev[l], cudaEventDisableTiming) == cudaSuccess;
-        if (!ok) { og_free(ctx); return OG_E_CUDA; }
-    }
     int32_t rc = mimc_init(ctx);
     if (rc != OG_OK) { og_free(ctx); return rc; }
     *out = ctx;
@@ -130,14 +116,6 @@ void og_free(og_ctx* ctx) {
     if (!ctx) return;
     cudaSetDevice(ctx->device);
     cudaDeviceSynchronize();
-    ctx->stream = ctx->main_stream ? ctx->main_stream : ctx->stream;
-    for (int l = 0; l < MAX_LANES; l++) {
-        if (ctx->lane_hi[l]) cudaStreamDestroy(ctx->lane_hi[l]);
-        if (ctx->lane_lo[l]) cudaStreamDestroy(ctx->lane_lo[l]);
-        if (ctx->lane_ev[l]) cudaEventDestroy(ctx->lane_ev[l]);
-    }
-    if (ctx->fork_ev) cudaEventDestroy(ctx->fork_ev);
-    if (ctx->acc_ev) cudaEventDestroy(ctx->acc_ev);
     for (int i = 0; i < N_SLOTS; i++) if (ctx->slot_ptr[i]) cudaFree(ctx->slot_ptr[i]);
     ntt_free_tables(ctx);
     if (ctx->g1_fixed) cudaFree(ctx->g1_fixed);
@@ -161,7 +139,7 @@ int32_t og_sync(og_ctx* ctx) {
 }
 int32_t og_stream(og_ctx* ctx, void** out_cuda_stream) {
     if (!ctx || !out_cuda_stream) return OG_E_INVALID;
-    *out_cuda_stream = (void*)ctx->main_stream;
+    *out_cuda_stream = (void*)ctx->stream;
     return OG_OK;
 }
 int32_t og_timer_start(og_ctx* ctx) {

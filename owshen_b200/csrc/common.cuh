@@ -13,7 +13,6 @@
 namespace og {
 
 constexpr int N_SLOTS = 64;
-constexpr int MAX_LANES = 2;   // chunks of a proving batch in flight at the same time (groth16.cu)
 
 struct NttTables;   // ntt.cu
 
@@ -22,16 +21,7 @@ struct NttTables;   // ntt.cu
 struct og_ctx {
     int device = 0;
     int sm_count = 148;
-    cudaStream_t stream = nullptr;        // the stream launches go to NOW (OG_LAUNCH); == main_stream outside a lane
-    cudaStream_t main_stream = nullptr;   // what og_sync / og_timer_* / the host-pointer copies use
-    // the batched prover keeps MAX_LANES chunks in flight: per lane one high-priority stream for the short
-    // latency-bound kernels (sort, scan, reduction, NTT, witness) and one low-priority stream for the long
-    // issue-bound bucket accumulation, so that the tails of one chunk run under the accumulation of the other
-    cudaStream_t lane_hi[og::MAX_LANES] = {nullptr}, lane_lo[og::MAX_LANES] = {nullptr};
-    cudaEvent_t lane_ev[og::MAX_LANES] = {nullptr}, fork_ev = nullptr;
-    cudaStream_t acc_stream = nullptr;    // when set, msm_buckets launches its accumulation kernel there
-    cudaEvent_t acc_ev = nullptr;
-    int lane = 0;                         // selects the per-lane scratch slots
+    cudaStream_t stream = nullptr;        // every launch and copy of the library (og_stream returns it)
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     uint64_t launches = 0;
     char err[512] = {0};
@@ -100,18 +90,9 @@ enum Slot {
     S_PR_WIT, S_PR_ABC, S_PR_SCALARS, S_PR_SORTED, S_PR_COUNTS, S_PR_OFFSETS, S_PR_CURSOR, S_PR_BUCKETS,
     S_PR_SEG, S_PR_SUMS, S_PR_OUT, S_PR_PUB, S_PR_MISC, S_PR_HEAVY,
     S_SETUP_A, S_SETUP_B, S_SETUP_C,
-    // lane 1 copies of the per-chunk prover scratch (same order as S_PR_ABC .. S_PR_HEAVY) and of S_MSM_MISC
-    S_L1_ABC, S_L1_SCALARS, S_L1_SORTED, S_L1_COUNTS, S_L1_OFFSETS, S_L1_CURSOR, S_L1_BUCKETS, S_L1_SEG, S_L1_HEAVY, S_L1_MSM_MISC,
-    S_PR_AFF, S_L1_AFF, S_MSM_AFF,
     S_COUNT
 };
 static_assert(S_COUNT <= N_SLOTS, "grow N_SLOTS");
-
-// `from` has produced what `to` is about to consume
-static inline cudaError_t stream_handoff(cudaEvent_t ev, cudaStream_t from, cudaStream_t to) {
-    cudaError_t e = cudaEventRecord(ev, from);
-    return e != cudaSuccess ? e : cudaStreamWaitEvent(to, ev, 0);
-}
 
 static inline bool aligned32(const void* p) { return (((uintptr_t)p) & 31) == 0; }
 

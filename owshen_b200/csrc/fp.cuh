@@ -399,14 +399,9 @@ struct alignas(32) Fp {
     OG_HD bool operator!=(const Fp& b) const { return !(*this == b); }
 
     OG_HD friend Fp operator*(const Fp& a, const Fp& b) { Fp r; mont_mul<P>(r.l, a.l, b.l); return r; }
-#if defined(OG_SQR_INTERLEAVED)
-    // A/B switch: squarings through the interleaved multiplier.  Round 1 built the G1 unit this way (its bucket kernel kept
-    // the accumulator in registers then and was register-bound: 248.9 vs 245.6 ms per 1024 proofs); with the accumulator in
-    // shared memory the wide squarer wins by 0.8 % (231.5 vs 233.3 ms, profiles/r2_small_ab.md) and every unit uses it
-    OG_HD Fp sqr() const { Fp r; mont_mul<P>(r.l, l, l); return r; }
-#else
+    // the wide squarer: with the bucket accumulators in shared memory it beats squaring through the interleaved multiplier by
+    // 0.8 % (231.5 vs 233.3 ms per 1024 proofs, profiles/r2_small_ab.md)
     OG_HD Fp sqr() const { Fp r; uint32_t T[16]; sqr_wide(T, l); mont_reduce_wide<P>(r.l, T); return r; }   // 36 + 64 products
-#endif
 
     // lazy forms for long dependent chains (MiMC): values in [0, 2p), no final subtraction (bounds at mont_mul_lazy)
     OG_HD static Fp mul_lazy(const Fp& a, const Fp& b) { Fp r; mont_mul_lazy<P>(r.l, a.l, b.l); return r; }

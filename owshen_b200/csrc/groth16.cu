@@ -323,59 +323,38 @@ void pk_info(const og_pk* pk, uint32_t* n_vars, uint32_t* n_pub, uint32_t* log_m
 }
 
 // ---- the prover ---------------------------------------------------------------------------------------------
-// A batch is cut into chunks of CB proofs; up to MAX_LANES chunks are in flight, each lane with its own scratch
-// and its own pair of streams (common.cuh): the short latency-bound kernels of one chunk (witness chains, sort,
-// scan, NTT, bucket reduction, final s*A) run under the issue-bound bucket accumulation of the other.
+// A batch is cut into chunks of CB proofs that run one after another on the context's stream and share one set of
+// chunk scratch.
 struct ChunkBufs {
     Fr *W, *rs_m, *abc, *ntt_tmp, *bsc, *csc;
     uint32_t *counts, *offsets, *cursor, *sorted, *heavy;
     G1XYZZ *bk1, *lvl1, *totA, *totC;
     G2XYZZ *bk2, *lvl2, *totB;
-    void *aff1, *aff2;                    // batched-affine scratch (nullptr = XYZZ accumulation): G1 MSMs / G2 MSM
     uint32_t w_stride, bsc_stride, csc_stride;
 };
 
-// experiment builds only (-DOG_EXPERIMENT_AFFINE, csrc/experiments/bucket_affine.cuh): OG_AFFINE bit 0 = batched-affine
-// accumulation for the G1 MSMs of the prover, bit 1 = for the G2 MSM.  The shipped library has no such path.
-#ifdef OG_EXPERIMENT_AFFINE
-static uint32_t affine_mode() { return env_u32("OG_AFFINE", 0); }
-#else
-static uint32_t affine_mode() { return 0; }
-#endif
-
-// W, rs_m and the per-proof totals cover the whole batch; everything else is per chunk of B proofs and per lane
-static int32_t alloc_chunk(og_ctx* ctx, const og_pk* pk, uint32_t batch, uint32_t B, int lane, ChunkBufs& b) {
+// W, rs_m and the per-proof totals cover the whole batch; everything else is per chunk of B proofs
+static int32_t alloc_chunk(og_ctx* ctx, const og_pk* pk, uint32_t batch, uint32_t B, ChunkBufs& b) {
     const uint32_t m = 1u << pk->log_m;
     b.w_stride = pk->n_vars + 2;
     b.bsc_stride = pk->nB;
     b.csc_stride = pk->nC;
     size_t max_pts = pk->nC > pk->nA ? pk->nC : pk->nA;
     size_t n_keys = (size_t)B * pk->max_nb;
-    auto S = [&](int id0, int id1) { return lane ? id1 : id0; };
     b.W = (Fr*)ctx->slot(S_PR_WIT, sizeof(Fr) * (size_t)batch * b.w_stride);
     b.rs_m = (Fr*)ctx->slot(S_PR_MISC, sizeof(Fr) * 2 * (size_t)batch);
-    b.abc = (Fr*)ctx->slot(S(S_PR_ABC, S_L1_ABC), sizeof(Fr) * (size_t)B * 3 * m * 2);
-    b.bsc = (Fr*)ctx->slot(S(S_PR_SCALARS, S_L1_SCALARS), sizeof(Fr) * (size_t)B * (b.bsc_stride + b.csc_stride));
-    b.sorted = (uint32_t*)ctx->slot(S(S_PR_SORTED, S_L1_SORTED), 4 * (size_t)B * max_pts * pk->max_windows);
-    b.counts = (uint32_t*)ctx->slot(S(S_PR_COUNTS, S_L1_COUNTS), 4 * n_keys);
-    b.offsets = (uint32_t*)ctx->slot(S(S_PR_OFFSETS, S_L1_OFFSETS), 4 * (n_keys + 1));
-    b.cursor = (uint32_t*)ctx->slot(S(S_PR_CURSOR, S_L1_CURSOR), 4 * n_keys);
-    b.heavy = (uint32_t*)ctx->slot(S(S_PR_HEAVY, S_L1_HEAVY), 4 * (2 * n_keys + 4));
-    b.bk2 = (G2XYZZ*)ctx->slot(S(S_PR_BUCKETS, S_L1_BUCKETS), sizeof(G2XYZZ) * n_keys);
-    b.lvl2 = (G2XYZZ*)ctx->slot(S(S_PR_SEG, S_L1_SEG), sizeof(G2XYZZ) * msm_lvl_elems(B, pk->max_nb));
+    b.abc = (Fr*)ctx->slot(S_PR_ABC, sizeof(Fr) * (size_t)B * 3 * m * 2);
+    b.bsc = (Fr*)ctx->slot(S_PR_SCALARS, sizeof(Fr) * (size_t)B * (b.bsc_stride + b.csc_stride));
+    b.sorted = (uint32_t*)ctx->slot(S_PR_SORTED, 4 * (size_t)B * max_pts * pk->max_windows);
+    b.counts = (uint32_t*)ctx->slot(S_PR_COUNTS, 4 * n_keys);
+    b.offsets = (uint32_t*)ctx->slot(S_PR_OFFSETS, 4 * (n_keys + 1));
+    b.cursor = (uint32_t*)ctx->slot(S_PR_CURSOR, 4 * n_keys);
+    b.heavy = (uint32_t*)ctx->slot(S_PR_HEAVY, 4 * (2 * n_keys + 4));
+    b.bk2 = (G2XYZZ*)ctx->slot(S_PR_BUCKETS, sizeof(G2XYZZ) * n_keys);
+    b.lvl2 = (G2XYZZ*)ctx->slot(S_PR_SEG, sizeof(G2XYZZ) * msm_lvl_elems(B, pk->max_nb));
     b.totA = (G1XYZZ*)ctx->slot(S_PR_SUMS, (sizeof(G1XYZZ) * 2 + sizeof(G2XYZZ)) * (size_t)batch);
     if (!b.W || !b.rs_m || !b.abc || !b.bsc || !b.sorted || !b.counts || !b.offsets || !b.cursor || !b.heavy || !b.bk2 || !b.lvl2 || !b.totA)
         return OG_E_NOMEM;
-    b.aff1 = b.aff2 = nullptr;
-    if (affine_mode()) {
-        size_t need = 0;
-        if (affine_mode() & 1) need = msm_aff_scratch_bytes_g1(n_keys);
-        if ((affine_mode() & 2) && msm_aff_scratch_bytes_g2((size_t)B * pk->nb[1]) > need) need = msm_aff_scratch_bytes_g2((size_t)B * pk->nb[1]);
-        void* a = ctx->slot(S(S_PR_AFF, S_L1_AFF), need);
-        if (!a) return OG_E_NOMEM;
-        if (affine_mode() & 1) b.aff1 = a;
-        if (affine_mode() & 2) b.aff2 = a;
-    }
     b.ntt_tmp = b.abc + (size_t)B * 3 * m;
     b.csc = b.bsc + (size_t)B * b.bsc_stride;
     b.bk1 = reinterpret_cast<G1XYZZ*>(b.bk2);       // the G1 and G2 MSMs of a chunk run one after another
@@ -395,7 +374,7 @@ static int32_t run_msm_g1(og_ctx* ctx, const og_pk* pk, int which, ChunkBufs& b,
     plan.montgomery = 1;
     uint32_t n_keys = B * pk->nb[which];
     OG_TRY(msm_sort_digits(ctx, plan, n_keys, b.counts, b.offsets, b.cursor, b.sorted));
-    return msm_buckets_g1(ctx, table, b.sorted, b.offsets, b.counts, B, pk->nb[which], (uint64_t)B * n_pts * pk->n_windows[which], b.bk1, b.lvl1, b.heavy, b.cursor, totals, b.aff1);
+    return msm_buckets_g1(ctx, table, b.sorted, b.offsets, b.counts, B, pk->nb[which], (uint64_t)B * n_pts * pk->n_windows[which], b.bk1, b.lvl1, b.heavy, b.cursor, totals);
 }
 static int32_t run_msm_g2(og_ctx* ctx, const og_pk* pk, int which, ChunkBufs& b, uint32_t B, const G2Affine* table, uint32_t n_pts,
                           const Fr* scalars, uint32_t stride, G2XYZZ* totals) {
@@ -407,7 +386,7 @@ static int32_t run_msm_g2(og_ctx* ctx, const og_pk* pk, int which, ChunkBufs& b,
     plan.montgomery = 1;
     uint32_t n_keys = B * pk->nb[which];
     OG_TRY(msm_sort_digits(ctx, plan, n_keys, b.counts, b.offsets, b.cursor, b.sorted));
-    return msm_buckets_g2(ctx, table, b.sorted, b.offsets, b.counts, B, pk->nb[which], (uint64_t)B * n_pts * pk->n_windows[which], b.bk2, b.lvl2, b.heavy, b.cursor, totals, b.aff2);
+    return msm_buckets_g2(ctx, table, b.sorted, b.offsets, b.counts, B, pk->nb[which], (uint64_t)B * n_pts * pk->n_windows[which], b.bk2, b.lvl2, b.heavy, b.cursor, totals);
 }
 
 // where a chunk's witness rows come from
@@ -459,7 +438,7 @@ static uint32_t chunk_limit(const og_pk* pk) {
     return (uint32_t)(lim < 1 ? 1 : lim);
 }
 
-// OG_CHUNK proofs per chunk (default 1024 = the whole BASELINE batch, ~28 GB of scratch per lane; profiles/r2_lanes_sweep.md), OG_LANES chunks in flight (default 2, 1 = serial)
+// OG_CHUNK proofs per chunk (default 1024 = the whole BASELINE batch, ~28 GB of scratch; profiles/r2_lanes_sweep.md)
 static uint32_t chunk_size(const og_pk* pk, uint32_t batch) {
     uint32_t c = env_u32("OG_CHUNK", 1024);
     if (c > chunk_limit(pk)) c = chunk_limit(pk);
@@ -468,33 +447,10 @@ static uint32_t chunk_size(const og_pk* pk, uint32_t batch) {
 
 static int32_t prove_batch(og_ctx* ctx, const og_pk* pk, const WitnessSource& src, uint32_t batch, const uint8_t* d_rs, uint8_t* d_proofs) {
     const uint32_t CB = chunk_size(pk, batch);
-    const uint32_t n_chunks = (batch + CB - 1) / CB;
-    uint32_t lanes = env_u32("OG_LANES", MAX_LANES);
-    if (lanes > (uint32_t)MAX_LANES) lanes = MAX_LANES;
-    if (lanes > n_chunks) lanes = n_chunks;
-    ChunkBufs bufs[MAX_LANES];
-    for (uint32_t l = 0; l < lanes; l++) OG_TRY(alloc_chunk(ctx, pk, batch, CB, (int)l, bufs[l]));
-    OG_TRY(ntt_prepare(ctx, pk->log_m));
-    cudaStream_t main_s = ctx->stream;
-    if (lanes <= 1) {
-        for (uint32_t off = 0; off < batch; off += CB) OG_TRY(prove_chunk(ctx, pk, bufs[0], src, off, batch - off < CB ? batch - off : CB, d_rs, d_proofs));
-        return OG_OK;
-    }
-    OG_CUDA(ctx, cudaEventRecord(ctx->fork_ev, main_s));
-    for (uint32_t l = 0; l < lanes; l++) OG_CUDA(ctx, cudaStreamWaitEvent(ctx->lane_hi[l], ctx->fork_ev, 0));
-    int32_t rc = OG_OK;
-    for (uint32_t c = 0; c < n_chunks && rc == OG_OK; c++) {
-        uint32_t l = c % lanes, off = c * CB;
-        ctx->lane = (int)l; ctx->stream = ctx->lane_hi[l]; ctx->acc_stream = ctx->lane_lo[l];
-        rc = prove_chunk(ctx, pk, bufs[l], src, off, batch - off < CB ? batch - off : CB, d_rs, d_proofs);
-    }
-    ctx->lane = 0; ctx->stream = main_s; ctx->acc_stream = nullptr;
-    // join: whatever was enqueued must finish before the caller's stream goes on (also on the error path)
-    for (uint32_t l = 0; l < lanes; l++) {
-        cudaError_t e = stream_handoff(ctx->lane_ev[l], ctx->lane_hi[l], main_s);
-        if (e != cudaSuccess && rc == OG_OK) { snprintf(ctx->err, sizeof(ctx->err), "lane join: %s", cudaGetErrorString(e)); rc = OG_E_CUDA; }
-    }
-    return rc;
+    ChunkBufs b;
+    OG_TRY(alloc_chunk(ctx, pk, batch, CB, b));
+    for (uint32_t off = 0; off < batch; off += CB) OG_TRY(prove_chunk(ctx, pk, b, src, off, batch - off < CB ? batch - off : CB, d_rs, d_proofs));
+    return OG_OK;
 }
 
 int32_t prove_withdraw_dev(og_ctx* ctx, const og_pk* pk, const uint8_t* d_null, const uint8_t* d_sec, const uint8_t* d_rec,
@@ -519,7 +475,7 @@ int32_t prove_witness_dev(og_ctx* ctx, const og_pk* pk, const uint8_t* d_wit, ui
 // debug / parity probe: d_j for one witness (canonical bytes on device in and out)
 int32_t h_evals_dev(og_ctx* ctx, const og_pk* pk, const uint8_t* d_wit, uint8_t* d_out) {
     ChunkBufs b;
-    OG_TRY(alloc_chunk(ctx, pk, 1, 1, 0, b));
+    OG_TRY(alloc_chunk(ctx, pk, 1, 1, b));
     const uint32_t m = 1u << pk->log_m, n_priv = pk->n_vars - pk->n_pub - 1;
     OG_LAUNCH(ctx, k_witness_in, (pk->n_vars + 127) / 128, 128, 0, d_wit, 1, pk->n_vars, b.w_stride, b.W, ctx->d_flag);
     CsrDev A{pk->a_ptr, pk->a_col, pk->a_val}, Bm{pk->b_ptr, pk->b_col, pk->b_val};

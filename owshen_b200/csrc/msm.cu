@@ -13,7 +13,6 @@
 // integer multiply-add pipe, not HBM: a G1 mixed add moves 64 B + 4 B and costs ~3.5k instructions.
 #include "msm.cuh"
 #include "glv.cuh"
-#include <stdlib.h>
 // Compiled twice: -DOG_MSM_G1 (G1 instantiations + the curve-independent sort) and -DOG_MSM_G2.
 #if !defined(OG_MSM_G1) && !defined(OG_MSM_G2)
 #error "compile msm.cu with -DOG_MSM_G1 or -DOG_MSM_G2"
@@ -246,7 +245,7 @@ int32_t msm_sort_digits(og_ctx* ctx, const DigitPlan& plan, uint32_t n_keys, uin
     else OG_LAUNCHN(ctx, "k_digits_count", k_digits<false>, grid, 256, 0, plan, d_counts, nullptr, nullptr, nullptr, ctx->d_flag);
     {   // offsets[n_keys] receives the grand total; cursor[k] = offsets[k] for the scatter
         uint32_t n_tiles = (n_keys + SCAN_TILE - 1) / SCAN_TILE;
-        OG_SLOT(ctx, tile_sums, uint32_t, ctx->lane ? S_L1_MSM_MISC : S_MSM_MISC, 4 * (size_t)n_tiles);
+        OG_SLOT(ctx, tile_sums, uint32_t, S_MSM_MISC, 4 * (size_t)n_tiles);
         OG_LAUNCH(ctx, k_scan_tiles, n_tiles, SCAN_THREADS, 0, d_counts, n_keys, tile_sums);
         OG_LAUNCH(ctx, k_scan_tile_sums, 1, SCAN_THREADS, 0, tile_sums, n_tiles, d_offsets + n_keys);
         OG_LAUNCH(ctx, k_scan_apply, n_tiles, SCAN_THREADS, 0, d_counts, n_keys, tile_sums, d_offsets, d_cursor);
@@ -321,25 +320,8 @@ struct SmAcc1 {
 // the two squarings of a mixed addition through ONE out-of-line copy of the wide squarer (8 registers in, 8 out): with the squarer
 // inlined twice next to eight inlined products the kernel outgrew the instruction cache (ncu: 12.7 % of the warp samples waiting
 // for instructions after the wide squarer replaced the interleaved one, profiles/r2_small_ab.md)
-#ifndef OG_SQR_CALL
-#define OG_SQR_CALL 1
-#endif
-#if OG_SQR_CALL
 static __device__ __noinline__ Fq fq_sqr_call(Fq a) { return a.sqr(); }
-#define OG_ACC_SQR(x) fq_sqr_call(x)
-#else
-#define OG_ACC_SQR(x) (x).sqr()
-#endif
-#if defined(OG_MUL_CALL) && OG_MUL_CALL      // A/B: the eight products out of line as well
-static __device__ __noinline__ Fq fq_mul_call(Fq a, Fq b) { return a * b; }
-#define OG_ACC_MUL(x, y) fq_mul_call((x), (y))
-#else
-#define OG_ACC_MUL(x, y) ((x) * (y))
-#endif
-#ifndef OG_ACC1_MINB
-#define OG_ACC1_MINB 8
-#endif
-__global__ void __launch_bounds__(128, OG_ACC1_MINB) k_bucket_acc_sm1(const Affine<Fq>* __restrict__ table, const uint32_t* __restrict__ sorted,
+__global__ void __launch_bounds__(128, 8) k_bucket_acc_sm1(const Affine<Fq>* __restrict__ table, const uint32_t* __restrict__ sorted,
                                                         const uint32_t* __restrict__ offsets, const uint32_t* __restrict__ counts,
                                                         uint32_t n_keys, uint32_t cap, XYZZ<Fq>* __restrict__ buckets,
                                                         uint32_t* __restrict__ heavy, const uint32_t* __restrict__ perm) {
@@ -363,22 +345,22 @@ __global__ void __launch_bounds__(128, OG_ACC1_MINB) k_bucket_acc_sm1(const Affi
         e = en;
         if (q.is_inf()) continue;
         if (inf) { A.st(0, q.x); A.st(1, q.y); A.st(2, Fq::one()); A.st(3, Fq::one()); inf = false; continue; }
-        Fq p = OG_ACC_MUL(q.x, A.ld(2)) - A.ld(0);
-        Fq r = OG_ACC_MUL(q.y, A.ld(3)) - A.ld(1);
+        Fq p = q.x * A.ld(2) - A.ld(0);
+        Fq r = q.y * A.ld(3) - A.ld(1);
         if (p.is_zero()) {
             if (r.is_zero()) { XYZZ<Fq> d = XYZZ<Fq>::dbl_affine(q); A.st(0, d.x); A.st(1, d.y); A.st(2, d.zz); A.st(3, d.zzz); }
             else inf = true;
             continue;
         }
         // ordered so that few temporaries are live at a time: zz and zzz are updated as soon as pp / ppp exist
-        Fq pp = OG_ACC_SQR(p);
-        A.st(2, OG_ACC_MUL(A.ld(2), pp));
-        Fq ppp = OG_ACC_MUL(p, pp);
-        A.st(3, OG_ACC_MUL(A.ld(3), ppp));
-        Fq q1 = OG_ACC_MUL(A.ld(0), pp);
-        Fq x3 = OG_ACC_SQR(r) - ppp - q1.dbl();
+        Fq pp = fq_sqr_call(p);
+        A.st(2, A.ld(2) * pp);
+        Fq ppp = p * pp;
+        A.st(3, A.ld(3) * ppp);
+        Fq q1 = A.ld(0) * pp;
+        Fq x3 = fq_sqr_call(r) - ppp - q1.dbl();
         A.st(0, x3);
-        A.st(1, OG_ACC_MUL(r, q1 - x3) - OG_ACC_MUL(A.ld(1), ppp));
+        A.st(1, r * (q1 - x3) - A.ld(1) * ppp);
     }
     buckets[key] = inf ? XYZZ<Fq>::inf() : XYZZ<Fq>{A.ld(0), A.ld(1), A.ld(2), A.ld(3)};
 }
@@ -534,10 +516,6 @@ __global__ void __launch_bounds__(32) k_heavy_combine(const XYZZ<F>* __restrict_
         __syncwarp();
     }
 }
-
-#ifdef OG_EXPERIMENT_AFFINE
-#include "experiments/bucket_affine.cuh"      // rejected in round 2 (profiles/r2_affine_ab.md); not in the shipped library
-#endif
 
 constexpr uint32_t RED_FAN_LOG2 = 3, RED_FAN = 1u << RED_FAN_LOG2;   // 8 children per parent: more threads, shorter chains
 // ---- 5: weighted reduction, RED_FAN children per parent -------------------------------------------------------
@@ -706,11 +684,8 @@ __global__ void __launch_bounds__(64) k_group_total(const XYZZ<F>* __restrict__ 
 // log2(n1) sums Q_k are independent tree reductions (one CTA each: a few strided additions per thread, then log2(threads) levels
 // in shared memory); one thread per group finishes with a Horner over the bits.  Depth ~16 + 28 group operations instead of ~120.
 constexpr uint32_t TAIL_THREADS = 128, TAIL_SLICE = 512;
-#ifndef OG_TAIL_MINB
-#define OG_TAIL_MINB 1
-#endif
 template <class F>
-__global__ void __launch_bounds__(TAIL_THREADS, OG_TAIL_MINB) k_tail_sums(const XYZZ<F>* __restrict__ R, const XYZZ<F>* __restrict__ T, uint32_t n1,
+__global__ void __launch_bounds__(TAIL_THREADS, 1) k_tail_sums(const XYZZ<F>* __restrict__ R, const XYZZ<F>* __restrict__ T, uint32_t n1,
                                                             uint32_t n_sums, uint32_t n_slices, XYZZ<F>* __restrict__ out) {
     __shared__ XYZZ<F> a[TAIL_THREADS];
     const uint32_t q = blockIdx.x, g = blockIdx.y, sl = blockIdx.z, tid = threadIdx.x;    // q = 0: sum T, 1: sum R, 2 + k: Q_k
@@ -763,8 +738,7 @@ __global__ void __launch_bounds__(TAIL_THREADS) k_tail_finish(const XYZZ<F>* __r
 template <class F>
 static int32_t msm_buckets(og_ctx* ctx, const Affine<F>* d_table, const uint32_t* d_sorted, const uint32_t* d_offsets,
                            const uint32_t* d_counts, uint32_t n_groups, uint32_t nb, uint64_t n_entries_max, XYZZ<F>* d_buckets,
-                           XYZZ<F>* d_lvl, uint32_t* d_heavy, uint32_t* d_perm, XYZZ<F>* d_totals, void* aff_scratch = nullptr,
-                           bool few_groups = false) {
+                           XYZZ<F>* d_lvl, uint32_t* d_heavy, uint32_t* d_perm, XYZZ<F>* d_totals, bool few_groups = false) {
     uint32_t n_keys = n_groups * nb;
     constexpr int HT = sizeof(F) == 32 ? 256 : 128;
     OG_CUDA(ctx, cudaMemsetAsync(d_heavy, 0, sizeof(uint32_t), ctx->stream));
@@ -773,29 +747,11 @@ static int32_t msm_buckets(og_ctx* ctx, const Affine<F>* d_table, const uint32_t
     // (skewed scalars: witness 0/1 values, short scalars whose top window has few distinct digits)
     uint64_t avg = n_entries_max / (n_keys ? n_keys : 1);
     uint32_t cap = (uint32_t)(4 * avg < 128 ? 128 : 4 * avg);
-#ifdef OG_EXPERIMENT_AFFINE
-    if (aff_scratch) {
-        OG_TRY((bucket_acc_affine<F>(ctx, d_table, d_sorted, d_offsets, d_counts, n_keys, cap, avg, d_buckets, d_heavy, d_perm, aff_scratch)));
-    } else
-#endif
-    {
-        // the long issue-bound kernel of the MSM: on the lane's low-priority stream when the prover runs chunks in flight
-        const char* kn = sizeof(F) == 32 ? "k_bucket_acc_g1" : "k_bucket_acc_g2";
-        unsigned grid = (n_keys + 127) / 128;
-        cudaStream_t hi = ctx->stream;
-        if (ctx->acc_stream) { OG_CUDA(ctx, stream_handoff(ctx->acc_ev, hi, ctx->acc_stream)); ctx->stream = ctx->acc_stream; }
-        int32_t rc = [&]() -> int32_t {
 #ifdef OG_MSM_G1
-            OG_LAUNCHN(ctx, kn, k_bucket_acc_sm1, grid, 128, 0, d_table, d_sorted, d_offsets, d_counts, n_keys, cap, d_buckets, d_heavy, d_perm);
+    OG_LAUNCHN(ctx, "k_bucket_acc_g1", k_bucket_acc_sm1, (n_keys + 127) / 128, 128, 0, d_table, d_sorted, d_offsets, d_counts, n_keys, cap, d_buckets, d_heavy, d_perm);
 #else
-            OG_LAUNCHN(ctx, kn, k_bucket_acc_sm, grid, 128, 0, d_table, d_sorted, d_offsets, d_counts, n_keys, cap, d_buckets, d_heavy, d_perm);
+    OG_LAUNCHN(ctx, "k_bucket_acc_g2", k_bucket_acc_sm, (n_keys + 127) / 128, 128, 0, d_table, d_sorted, d_offsets, d_counts, n_keys, cap, d_buckets, d_heavy, d_perm);
 #endif
-            return OG_OK;
-        }();
-        ctx->stream = hi;
-        OG_TRY(rc);
-        if (ctx->acc_stream) OG_CUDA(ctx, stream_handoff(ctx->acc_ev, ctx->acc_stream, hi));
-    }
     {
         // segment length: long enough that the segment sums of ALL heavy buckets fit in the (still unused) reduction scratch
         // (at most n_keys / 4 heavy buckets, since each holds more than 4 x the average load)
@@ -814,42 +770,35 @@ static int32_t msm_buckets(og_ctx* ctx, const Affine<F>* d_table, const uint32_t
     const XYZZ<F>* U_in = nullptr;
     uint32_t n_in = nb, w_log2 = 0;
     int pp = 0;
-    // level 0 (raw buckets) is most of the work: a wider fan there spends fewer additions per bucket (2 - 1/fan)
-    // and leaves less for the levels above, at the price of longer serial chains; OG_RED_FAN0 = 3, 4 or 5
-    static const uint32_t fan0 = [] { const char* v = getenv("OG_RED_FAN0"); int x = v ? atoi(v) : 0; return (uint32_t)(x >= 3 && x <= 5 ? x : RED_FAN_LOG2); }();
     do {
-        uint32_t fan_log2 = U_in ? RED_FAN_LOG2 : fan0;
-        uint32_t n_out = (n_in + (1u << fan_log2) - 1) >> fan_log2;
+        uint32_t n_out = (n_in + RED_FAN - 1) >> RED_FAN_LOG2;
         uint32_t threads = n_groups * n_out;
         const char* rn = sizeof(F) == 32 ? "k_reduce_level_g1" : "k_reduce_level_g2";
         // G1: running sums in registers, group operations out of line; G2: running sums in shared memory (profiles/r2_small_ab.md;
         // the losing combination of each was removed from the library after the measurement)
         if constexpr (RED_SM_DEFAULT<F>) {
-            if (U_in) { auto k = k_reduce_level_sm<F, true>; OG_LAUNCHN(ctx, rn, k, (threads + 63) / 64, 64, 0, S_in, U_in, n_in, n_out, n_groups, w_log2, fan_log2, bufS[pp], bufU[pp]); }
-            else { auto k = k_reduce_level_sm<F, false>; OG_LAUNCHN(ctx, rn, k, (threads + 63) / 64, 64, 0, S_in, U_in, n_in, n_out, n_groups, w_log2, fan_log2, bufS[pp], bufU[pp]); }
+            if (U_in) { auto k = k_reduce_level_sm<F, true>; OG_LAUNCHN(ctx, rn, k, (threads + 63) / 64, 64, 0, S_in, U_in, n_in, n_out, n_groups, w_log2, RED_FAN_LOG2, bufS[pp], bufU[pp]); }
+            else { auto k = k_reduce_level_sm<F, false>; OG_LAUNCHN(ctx, rn, k, (threads + 63) / 64, 64, 0, S_in, U_in, n_in, n_out, n_groups, w_log2, RED_FAN_LOG2, bufS[pp], bufU[pp]); }
         } else {
-            if (U_in) { auto k = k_reduce_level<F, true>; OG_LAUNCHN(ctx, rn, k, (threads + 63) / 64, 64, 0, S_in, U_in, n_in, n_out, n_groups, w_log2, fan_log2, bufS[pp], bufU[pp]); }
-            else { auto k = k_reduce_level<F, false>; OG_LAUNCHN(ctx, rn, k, (threads + 63) / 64, 64, 0, S_in, U_in, n_in, n_out, n_groups, w_log2, fan_log2, bufS[pp], bufU[pp]); }
+            if (U_in) { auto k = k_reduce_level<F, true>; OG_LAUNCHN(ctx, rn, k, (threads + 63) / 64, 64, 0, S_in, U_in, n_in, n_out, n_groups, w_log2, RED_FAN_LOG2, bufS[pp], bufU[pp]); }
+            else { auto k = k_reduce_level<F, false>; OG_LAUNCHN(ctx, rn, k, (threads + 63) / 64, 64, 0, S_in, U_in, n_in, n_out, n_groups, w_log2, RED_FAN_LOG2, bufS[pp], bufU[pp]); }
         }
         S_in = bufS[pp]; U_in = bufU[pp];
         pp ^= 1;
         n_in = n_out;
-        w_log2 += fan_log2;
-        if (few_groups && w_log2 == fan_log2 && n_in >= 64 && (n_in & (n_in - 1)) == 0) {
+        w_log2 += RED_FAN_LOG2;
+        if (few_groups && w_log2 == RED_FAN_LOG2 && n_in >= 64 && (n_in & (n_in - 1)) == 0) {
             // one-shot MSM: everything above level 0 as independent tree sums + one Horner per group (5b above)
-            static const bool tail = [] { const char* v = getenv("OG_MSM_TAIL"); return !(v && v[0] == '0' && v[1] == 0); }();
-            if (tail) {
-                uint32_t n_bits = 0;
-                while ((1u << n_bits) < n_in) n_bits++;
-                const uint32_t n_sums = n_bits + 2, n_slices = (n_in + TAIL_SLICE - 1) / TAIL_SLICE;
-                if (n_sums * n_slices <= TAIL_THREADS) {
-                    XYZZ<F>* partials = bufS[pp];                           // the other ping-pong buffer: n_groups * n_in / 8 + 16 >= n_groups * n_sums * n_slices
-                    OG_LAUNCHN(ctx, sizeof(F) == 32 ? "k_tail_sums_g1" : "k_tail_sums_g2", k_tail_sums<F>, dim3(n_sums, n_groups, n_slices), TAIL_THREADS, 0,
-                               S_in, U_in, n_in, n_sums, n_slices, partials);
-                    OG_LAUNCHN(ctx, sizeof(F) == 32 ? "k_tail_finish_g1" : "k_tail_finish_g2", k_tail_finish<F>, n_groups, TAIL_THREADS, 0, partials, n_sums, n_slices,
-                               w_log2, d_totals);
-                    return OG_OK;
-                }
+            uint32_t n_bits = 0;
+            while ((1u << n_bits) < n_in) n_bits++;
+            const uint32_t n_sums = n_bits + 2, n_slices = (n_in + TAIL_SLICE - 1) / TAIL_SLICE;
+            if (n_sums * n_slices <= TAIL_THREADS) {
+                XYZZ<F>* partials = bufS[pp];                           // the other ping-pong buffer: n_groups * n_in / 8 + 16 >= n_groups * n_sums * n_slices
+                OG_LAUNCHN(ctx, sizeof(F) == 32 ? "k_tail_sums_g1" : "k_tail_sums_g2", k_tail_sums<F>, dim3(n_sums, n_groups, n_slices), TAIL_THREADS, 0,
+                           S_in, U_in, n_in, n_sums, n_slices, partials);
+                OG_LAUNCHN(ctx, sizeof(F) == 32 ? "k_tail_finish_g1" : "k_tail_finish_g2", k_tail_finish<F>, n_groups, TAIL_THREADS, 0, partials, n_sums, n_slices,
+                           w_log2, d_totals);
+                return OG_OK;
             }
         }
     } while (n_in > 1);
@@ -860,27 +809,17 @@ static int32_t msm_buckets(og_ctx* ctx, const Affine<F>* d_table, const uint32_t
 #ifdef OG_MSM_G1
 int32_t msm_buckets_g1(og_ctx* ctx, const G1Affine* d_table, const uint32_t* d_sorted, const uint32_t* d_offsets,
                        const uint32_t* d_counts, uint32_t n_groups, uint32_t nb, uint64_t n_entries_max, G1XYZZ* d_buckets,
-                       G1XYZZ* d_lvl, uint32_t* d_heavy, uint32_t* d_perm, G1XYZZ* d_totals, void* aff_scratch) {
-    return msm_buckets<Fq>(ctx, d_table, d_sorted, d_offsets, d_counts, n_groups, nb, n_entries_max, d_buckets, d_lvl, d_heavy, d_perm, d_totals, aff_scratch);
+                       G1XYZZ* d_lvl, uint32_t* d_heavy, uint32_t* d_perm, G1XYZZ* d_totals) {
+    return msm_buckets<Fq>(ctx, d_table, d_sorted, d_offsets, d_counts, n_groups, nb, n_entries_max, d_buckets, d_lvl, d_heavy, d_perm, d_totals);
 }
-#ifdef OG_EXPERIMENT_AFFINE
-size_t msm_aff_scratch_bytes_g1(uint64_t n_keys) { return aff_scratch_bytes_t<Fq>(n_keys); }
-#else
-size_t msm_aff_scratch_bytes_g1(uint64_t) { return 0; }
-#endif
 #endif  // OG_MSM_G1
 
 #ifdef OG_MSM_G2
 int32_t msm_buckets_g2(og_ctx* ctx, const G2Affine* d_table, const uint32_t* d_sorted, const uint32_t* d_offsets,
                        const uint32_t* d_counts, uint32_t n_groups, uint32_t nb, uint64_t n_entries_max, G2XYZZ* d_buckets,
-                       G2XYZZ* d_lvl, uint32_t* d_heavy, uint32_t* d_perm, G2XYZZ* d_totals, void* aff_scratch) {
-    return msm_buckets<Fq2>(ctx, d_table, d_sorted, d_offsets, d_counts, n_groups, nb, n_entries_max, d_buckets, d_lvl, d_heavy, d_perm, d_totals, aff_scratch);
+                       G2XYZZ* d_lvl, uint32_t* d_heavy, uint32_t* d_perm, G2XYZZ* d_totals) {
+    return msm_buckets<Fq2>(ctx, d_table, d_sorted, d_offsets, d_counts, n_groups, nb, n_entries_max, d_buckets, d_lvl, d_heavy, d_perm, d_totals);
 }
-#ifdef OG_EXPERIMENT_AFFINE
-size_t msm_aff_scratch_bytes_g2(uint64_t n_keys) { return aff_scratch_bytes_t<Fq2>(n_keys); }
-#else
-size_t msm_aff_scratch_bytes_g2(uint64_t) { return 0; }
-#endif
 #endif  // OG_MSM_G2
 
 
@@ -1000,9 +939,8 @@ static int32_t msm_dev(og_ctx* ctx, const uint8_t* d_points, const uint8_t* d_sc
     if (!aligned32(d_points) || !aligned32(d_scalars)) return OG_E_INVALID;
     if (n == 0) { OG_CUDA(ctx, cudaMemsetAsync(d_out, 0, PB, ctx->stream)); return OG_OK; }
     // G1: GLV halves the scalar length (2n points, 127-bit scalars): same bucket additions, half the windows to reduce and half
-    // the sequential doublings of the Horner (OG_GLV=0 switches it off for A/B)
-    static const bool glv_on = [] { const char* v = getenv("OG_GLV"); return !(v && v[0] == '0' && v[1] == 0); }();
-    const bool glv = sizeof(F) == 32 && glv_on && n >= 1024;
+    // the sequential doublings of the Horner
+    const bool glv = sizeof(F) == 32 && n >= 1024;
     const uint64_t n_in = n;
     if (glv) n = 2 * n;
     uint32_t c = pick_window(n), W = glv ? (128 + c - 1) / c : msm_windows(c), nb = 1u << (c - 1);
@@ -1034,14 +972,7 @@ static int32_t msm_dev(og_ctx* ctx, const uint8_t* d_points, const uint8_t* d_sc
     plan.key_stride_problem = 0; plan.key_stride_window = 1; plan.tidx_window_stride = 0;
     plan.montgomery = 0;
     OG_TRY(msm_sort_digits(ctx, plan, n_keys, counts, offsets, cursor, sorted));
-    void* aff = nullptr;
-#ifdef OG_EXPERIMENT_AFFINE
-    {   // OG_AFFINE_ONESHOT=1 routes one-shot MSMs through the experiment so that the edge-case tests exercise it
-        const char* v = getenv("OG_AFFINE_ONESHOT");
-        if (v && atoi(v) > 0) { aff = ctx->slot(S_MSM_AFF, aff_scratch_bytes_t<F>(n_keys)); if (!aff) return OG_E_NOMEM; }
-    }
-#endif
-    OG_TRY((msm_buckets<F>(ctx, pts, sorted, offsets, counts, W, nb, n * W, buckets, lvl, heavy, cursor, totals, aff, true)));
+    OG_TRY((msm_buckets<F>(ctx, pts, sorted, offsets, counts, W, nb, n * W, buckets, lvl, heavy, cursor, totals, true)));
     OG_LAUNCH(ctx, k_horner<F>, 1, 128, 0, totals, W, c, d_out);
     return OG_OK;
 }

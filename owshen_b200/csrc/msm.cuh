@@ -35,14 +35,10 @@ int32_t msm_sort_digits(og_ctx* ctx, const DigitPlan& plan, uint32_t n_keys, uin
 // d_perm: n_keys u32 scratch (the sort's cursor array may be reused); result: d_totals[n_groups].
 int32_t msm_buckets_g1(og_ctx* ctx, const G1Affine* d_table, const uint32_t* d_sorted, const uint32_t* d_offsets,
                        const uint32_t* d_counts, uint32_t n_groups, uint32_t nb, uint64_t n_entries_max, G1XYZZ* d_buckets,
-                       G1XYZZ* d_lvl, uint32_t* d_heavy, uint32_t* d_perm, G1XYZZ* d_totals, void* aff_scratch = nullptr);
+                       G1XYZZ* d_lvl, uint32_t* d_heavy, uint32_t* d_perm, G1XYZZ* d_totals);
 int32_t msm_buckets_g2(og_ctx* ctx, const G2Affine* d_table, const uint32_t* d_sorted, const uint32_t* d_offsets,
                        const uint32_t* d_counts, uint32_t n_groups, uint32_t nb, uint64_t n_entries_max, G2XYZZ* d_buckets,
-                       G2XYZZ* d_lvl, uint32_t* d_heavy, uint32_t* d_perm, G2XYZZ* d_totals, void* aff_scratch = nullptr);
-// aff_scratch: experiment builds only (-DOG_EXPERIMENT_AFFINE): non-null selects the rejected batched-affine accumulation
-// (csrc/experiments/bucket_affine.cuh, profiles/r2_affine_ab.md); the shipped library ignores it and the sizes are 0
-size_t msm_aff_scratch_bytes_g1(uint64_t n_keys);
-size_t msm_aff_scratch_bytes_g2(uint64_t n_keys);
+                       G2XYZZ* d_lvl, uint32_t* d_heavy, uint32_t* d_perm, G2XYZZ* d_totals);
 static inline size_t msm_lvl_elems(uint32_t n_groups, uint32_t nb) { return 4 * ((size_t)n_groups * ((nb + 7) / 8) + 16); }   // RED_FAN = 8
 
 // one-shot MSMs on device buffers holding boundary bytes (affine points, canonical scalars)

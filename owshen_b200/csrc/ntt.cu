@@ -14,7 +14,6 @@
 // One table per size serves everything: T2[j] = omega_{2n}^j (j < n): coset factors are T2[j],
 // stage twiddles are omega_n^e = T2[2e], inverses are -T2[n - j].
 #include "ntt.cuh"
-#include <stdlib.h>
 
 namespace og {
 
@@ -55,30 +54,7 @@ struct PassPlan {
     uint32_t first, last, inverse, coset;
     uint32_t fold;      // 1: inverse transform whose 1/n is left to the next transform; 2: forward coset transform that applies it
                         // (its coset factors come from t2n = t2 / n): one product per element fewer for the pair (groth16.cu)
-    uint32_t tma;       // intermediate buffers hold elements with bit 2 of their index set with the two 16-byte halves swapped, and
-                        // non-first passes fetch their tile with cp.async.bulk (see k_ntt_pass2)
 };
-
-// ---- TMA bulk copies (cp.async.bulk, global -> shared, completion on an mbarrier) ---------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void* dst_smem, const void* src_gmem, uint32_t bytes, uint64_t* bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(smem_u32(dst_smem)), "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-    uint32_t ok;
-    do {
-        asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
-                     : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-    } while (!ok);
-}
 
 __device__ __forceinline__ uint32_t bitrev(uint32_t x, uint32_t bits) { return __brev(x) >> (32 - bits); }
 
@@ -101,10 +77,6 @@ __device__ __forceinline__ void sm_put(uint4* sm, uint32_t e, const Fr& v) {
     sm[sw_chunk(e, 1)] = make_uint4(v.l[4], v.l[5], v.l[6], v.l[7]);
 }
 
-// TMA (P.tma): the XOR swizzle only ever swaps the two 16-byte halves of elements whose index has bit 2 set, and in the
-// non-first passes a tile is made of 256-byte runs of 8 consecutive elements -- so when the PREVIOUS pass stores those
-// elements with their halves swapped, the tile in shared memory is a byte-for-byte copy of its runs in global memory, and
-// one warp can fetch it with 256-byte cp.async.bulk copies that complete on an mbarrier while no thread issues a load.
 // 3 resident CTAs of 256 threads per SM (80 registers): measured 35.7 -> 31.9 ms per 1024 proofs against 2 CTAs,
 // 4 CTAs (64 registers) was equal
 __global__ void __launch_bounds__(256, 3) k_ntt_pass2(PassPlan P, const Fr* __restrict__ in, Fr* __restrict__ out,
@@ -121,33 +93,20 @@ __global__ void __launch_bounds__(256, 3) k_ntt_pass2(PassPlan P, const Fr* __re
     Fr* dst = out + (size_t)blockIdx.y * n;
     const uint32_t lmask = (1u << P.L) - 1;
 
-    if (P.tma && !P.first) {                            // P.L == 3: 2^K runs of 256 bytes
-        __shared__ uint64_t bar;
-        if (threadIdx.x == 0) mbar_init(&bar, 1);
-        __syncthreads();
-        if (threadIdx.x < 32) {
-            if (threadIdx.x == 0) mbar_expect_tx(&bar, tile * (uint32_t)sizeof(Fr));
-            __syncwarp();
-            for (uint32_t k = threadIdx.x; k < (1u << P.K); k += 32)
-                bulk_g2s(smem_raw + 256u * k, src + (base | (k << B0)), 256u, &bar);
+    for (uint32_t e = threadIdx.x; e < tile; e += blockDim.x) {
+        uint32_t lo = e & lmask, k = e >> P.L;
+        uint32_t i = base | (k << B0) | lo;
+        Fr v;
+        if (P.first) {
+            uint32_t j = bitrev(i, P.log_n);
+            v = src[j];
+            if (P.coset && !P.inverse) v = v * (P.fold == 2 ? t2n[j] : t2[j]);
+        } else {
+            v = src[i];
         }
-        mbar_wait(&bar, 0);
-    } else {
-        for (uint32_t e = threadIdx.x; e < tile; e += blockDim.x) {
-            uint32_t lo = e & lmask, k = e >> P.L;
-            uint32_t i = base | (k << B0) | lo;
-            Fr v;
-            if (P.first) {
-                uint32_t j = bitrev(i, P.log_n);
-                v = src[j];
-                if (P.coset && !P.inverse) v = v * (P.fold == 2 ? t2n[j] : t2[j]);
-            } else {
-                v = src[i];
-            }
-            sm_put(sm, e, v);
-        }
-        __syncthreads();
+        sm_put(sm, e, v);
     }
+    __syncthreads();
 
     uint32_t q = 1;
     for (; q + 1 <= P.K; q += 2) {                      // two levels per barrier
@@ -203,14 +162,7 @@ __global__ void __launch_bounds__(256, 3) k_ntt_pass2(PassPlan P, const Fr* __re
             if (P.fold != 1) v = v * n_inv;
             if (P.coset) v = v * tw2(t2, n, i, true);
         }
-        if (P.tma && !P.last) {                         // intermediate buffer: halves swapped where bit 2 of the index is set
-            uint4* q4 = reinterpret_cast<uint4*>(dst + i);
-            const uint32_t sw = (i >> 2) & 1;
-            q4[sw] = make_uint4(v.l[0], v.l[1], v.l[2], v.l[3]);
-            q4[sw ^ 1] = make_uint4(v.l[4], v.l[5], v.l[6], v.l[7]);
-        } else {
-            dst[i] = v;
-        }
+        dst[i] = v;
     }
 }
 
@@ -242,8 +194,6 @@ static int32_t get_tables(og_ctx* ctx, uint32_t log_n, NttTables** out) {
     return OG_OK;
 }
 
-int32_t ntt_prepare(og_ctx* ctx, uint32_t log_n) { NttTables* T; return get_tables(ctx, log_n, &T); }
-
 void ntt_free_tables(og_ctx* ctx) {
     for (int i = 0; i < 32; i++)
         if (ctx->ntt[i]) { cudaFree(ctx->ntt[i]->d_t2); cudaFree(ctx->ntt[i]->d_t2n); delete ctx->ntt[i]; ctx->ntt[i] = nullptr; }
@@ -265,7 +215,7 @@ int32_t ntt_mont_dev(og_ctx* ctx, Fr* data, Fr* tmp, uint32_t log_n, uint32_t ba
     uint32_t done = 0;
     while (done < log_n) {
         PassPlan p;
-        p.log_n = log_n; p.s0 = done + 1; p.inverse = inverse; p.coset = coset; p.first = (done == 0); p.last = 0; p.tma = 0; p.fold = (uint32_t)fold;
+        p.log_n = log_n; p.s0 = done + 1; p.inverse = inverse; p.coset = coset; p.first = (done == 0); p.last = 0; p.fold = (uint32_t)fold;
         if (done == 0) { p.K = log_n < 10 ? log_n : 10; p.L = 0; }
         else {
             p.L = done < 3 ? done : 3;
@@ -278,10 +228,6 @@ int32_t ntt_mont_dev(og_ctx* ctx, Fr* data, Fr* tmp, uint32_t log_n, uint32_t ba
         plans[np++] = p;
     }
     plans[np - 1].last = 1;
-    // OG_NTT_TMA=1: intermediates pre-swizzled + TMA bulk tile loads in the non-first passes.  Measured equal in the prover (32.4 vs
-    // 32.4 ms per step) and 0.6-3.6 % slower standalone (profiles/r2_ntt_tma_ab.md), hence not the default
-    const int use_tma = [] { const char* e = getenv("OG_NTT_TMA"); return e ? atoi(e) : 0; }();     // read per call: tests toggle it
-    for (int i = 0; i < np; i++) plans[i].tma = (use_tma && np > 1) ? 1 : 0;
     for (int i = 0; i < np; i++) {
         const PassPlan& p = plans[i];
         const Fr* src = (i == 0) ? data : tmp;

@@ -9,7 +9,5 @@ namespace og {
 // a, b, c) can leave the 1/n to the coset factors of the second one: fold = 1 on the inverse (plain, non-coset) call, fold = 2 on
 // the forward coset call -- one product per element fewer for the pair.
 int32_t ntt_mont_dev(og_ctx* ctx, Fr* data, Fr* tmp, uint32_t log_n, uint32_t batch, int inverse, int coset, int fold = 0);
-// builds the twiddle table of size 2^log_n on the current stream if it does not exist yet (call before forking lanes)
-int32_t ntt_prepare(og_ctx* ctx, uint32_t log_n);
 void ntt_free_tables(og_ctx* ctx);
 }  // namespace og

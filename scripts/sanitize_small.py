@@ -29,10 +29,10 @@ ctx.bjj_verify_batch(fr(4), bytes(4), fr(4), fr(12))
 msgs = fr(4)
 pkx, odd, sigs, st = ctx.bjj_sign_batch(fr(4), fr(4), msgs)                            # window-table fixed-base path
 assert list(ctx.bjj_verify_batch(pkx, odd, msgs, sigs)) == [1] * 4
-# round 2 kernels: tree append, lanes (two chunks in flight), G2 heavy buckets, shared-memory G2 reduction, cooperative Horner
+# round 2 kernels: tree append, a batch in several chunks, G2 heavy buckets, shared-memory G2 reduction, cooperative Horner
 t = ob.MerkleTree(ctx, 5)
 t.insert_batch([1, 2, 3]); t.insert(4); t.insert_batch(list(range(5, 16))); t.rollback(6); t.pop_batch()
-os.environ["OG_CHUNK"] = "2"; os.environ["OG_LANES"] = "2"
+os.environ["OG_CHUNK"] = "2"
 b = 5
 proofs, pub = ob.prove(PK, fr(b), fr(b), fr(b), fr(b), [rng.randrange(2) for _ in range(b)], fr(2 * b))
 assert all(ob.verify(vk, pub[96 * i:96 * i + 96], proofs[256 * i:256 * i + 256]) for i in range(b))
@@ -40,7 +40,7 @@ p2 = ctx.g2_generator_mul(fr(1)) * 300
 ctx.msm_g2(p2, (5).to_bytes(32, "little") * 300)
 # later in round 2: reduction tail of one-shot MSMs (k_tail_sums / k_tail_finish need >= 512 buckets per window, i.e. >= 2^13 points),
 # three-barrier Horner, lazy MiMC chain (covered by merkle_paths above)
-os.environ.pop("OG_CHUNK"); os.environ.pop("OG_LANES")
+os.environ.pop("OG_CHUNK")
 pts = ctx.g1_generator_mul(fr(8192)); ctx.msm_g1(pts, fr(8192))
 pts = ctx.g2_generator_mul(fr(8192)); ctx.msm_g2(pts, fr(8192))
 PK.close(); ctx.close()
