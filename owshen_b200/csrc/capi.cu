@@ -72,6 +72,73 @@ int32_t check_flag(og_ctx* ctx) {
 #define H2D(ctx, dst, src, bytes) OG_CUDA(ctx, cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, (ctx)->stream))
 #define D2H(ctx, dst, src, bytes) OG_CUDA(ctx, cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, (ctx)->stream))
 
+// ---- the G1 / G2 entry points, written once over the coordinate field F (Fq: G1, Fq2: G2) --------------------------
+// A point crosses the boundary as 2 * sizeof(F) bytes (x, y canonical), the size of its affine Montgomery form.
+template <class F>
+static int32_t msm_dev_entry(og_ctx* ctx, const uint8_t* d_points, const uint8_t* d_scalars, uint64_t n, uint8_t* d_out) {
+    OG_ENTER(ctx);
+    if (!ctx || !d_out || (n && (!d_points || !d_scalars))) return OG_E_INVALID;
+    return msm_dev<F>(ctx, d_points, d_scalars, n, d_out);
+}
+template <class F>
+static int32_t msm_host_entry(og_ctx* ctx, const uint8_t* points, const uint8_t* scalars, uint64_t n, uint8_t* out) {
+    constexpr uint64_t PB = sizeof(Affine<F>);
+    OG_ENTER(ctx);
+    if (!ctx || !out || (n && (!points || !scalars))) return OG_E_INVALID;
+    OG_SLOT(ctx, dp, uint8_t, S_IO_A, PB * n);
+    OG_SLOT(ctx, ds, uint8_t, S_IO_B, 32 * n);
+    OG_SLOT(ctx, dout, uint8_t, S_IO_C, PB);
+    OG_TRY(clear_flag(ctx));
+    if (n) { H2D(ctx, dp, points, PB * n); H2D(ctx, ds, scalars, 32 * n); }
+    OG_TRY(msm_dev<F>(ctx, dp, ds, n, dout));
+    D2H(ctx, out, dout, PB);
+    return check_flag(ctx);
+}
+template <class F>
+static int32_t sum_host_entry(og_ctx* ctx, const uint8_t* points, uint64_t n, uint8_t* out) {
+    constexpr uint64_t PB = sizeof(Affine<F>);
+    OG_ENTER(ctx);
+    if (!ctx || !out || (n && !points)) return OG_E_INVALID;
+    OG_SLOT(ctx, dp, uint8_t, S_IO_A, PB * n);
+    OG_SLOT(ctx, dout, uint8_t, S_IO_C, PB);
+    OG_TRY(clear_flag(ctx));
+    if (n) H2D(ctx, dp, points, PB * n);
+    OG_TRY(sum_points_dev<F>(ctx, dp, n, dout));
+    D2H(ctx, out, dout, PB);
+    return check_flag(ctx);
+}
+template <class F>
+static int32_t sum_dev_entry(og_ctx* ctx, const uint8_t* d_points, uint64_t n, uint8_t* d_out) {
+    OG_ENTER(ctx);
+    if (!d_out || (n && !d_points)) return OG_E_INVALID;
+    return sum_points_dev<F>(ctx, d_points, n, d_out);
+}
+template <class F>
+static int32_t generator_mul_dev_entry(og_ctx* ctx, const uint8_t* d_scalars, uint64_t n, uint8_t* d_out_points) {
+    OG_ENTER(ctx);
+    if (n && (!d_scalars || !d_out_points)) return OG_E_INVALID;
+    if (n == 0) return OG_OK;
+    OG_SLOT(ctx, dp, Affine<F>, S_IO_B, sizeof(Affine<F>) * n);
+    OG_TRY(fixed_base_mul(ctx, d_scalars, n, dp));
+    return points_to_bytes(ctx, dp, n, d_out_points);
+}
+template <class F>
+static int32_t generator_mul_host_entry(og_ctx* ctx, const uint8_t* scalars, uint64_t n, uint8_t* out_points) {
+    constexpr uint64_t PB = sizeof(Affine<F>);
+    OG_ENTER(ctx);
+    if (!ctx || (n && (!scalars || !out_points))) return OG_E_INVALID;
+    if (n == 0) return OG_OK;
+    OG_SLOT(ctx, ds, uint8_t, S_IO_A, 32 * n);
+    OG_SLOT(ctx, dp, Affine<F>, S_IO_B, sizeof(Affine<F>) * n);
+    OG_SLOT(ctx, dout, uint8_t, S_IO_C, PB * n);
+    OG_TRY(clear_flag(ctx));
+    H2D(ctx, ds, scalars, 32 * n);
+    OG_TRY(fixed_base_mul(ctx, ds, n, dp));
+    OG_TRY(points_to_bytes(ctx, dp, n, dout));
+    D2H(ctx, out_points, dout, PB * n);
+    return check_flag(ctx);
+}
+
 extern "C" {
 
 int32_t og_abi_version(void) { return 1; }
@@ -618,117 +685,35 @@ int32_t og_bjj_sign_batch(og_ctx* ctx, const uint8_t* secret_keys, const uint8_t
 
 // ---- MSM --------------------------------------------------------------------------------------------------
 int32_t og_msm_g1_dev(og_ctx* ctx, const uint8_t* d_points, const uint8_t* d_scalars, uint64_t n, uint8_t* d_out64) {
-    OG_ENTER(ctx);
-    if (!ctx || !d_out64 || (n && (!d_points || !d_scalars))) return OG_E_INVALID;
-    return msm_g1_dev(ctx, d_points, d_scalars, n, d_out64);
+    return msm_dev_entry<Fq>(ctx, d_points, d_scalars, n, d_out64);
 }
 int32_t og_msm_g2_dev(og_ctx* ctx, const uint8_t* d_points, const uint8_t* d_scalars, uint64_t n, uint8_t* d_out128) {
-    OG_ENTER(ctx);
-    if (!ctx || !d_out128 || (n && (!d_points || !d_scalars))) return OG_E_INVALID;
-    return msm_g2_dev(ctx, d_points, d_scalars, n, d_out128);
+    return msm_dev_entry<Fq2>(ctx, d_points, d_scalars, n, d_out128);
 }
 int32_t og_msm_g1(og_ctx* ctx, const uint8_t* points, const uint8_t* scalars, uint64_t n, uint8_t* out64) {
-    OG_ENTER(ctx);
-    if (!ctx || !out64 || (n && (!points || !scalars))) return OG_E_INVALID;
-    OG_SLOT(ctx, dp, uint8_t, S_IO_A, 64 * n);
-    OG_SLOT(ctx, ds, uint8_t, S_IO_B, 32 * n);
-    OG_SLOT(ctx, dout, uint8_t, S_IO_C, 64);
-    OG_TRY(clear_flag(ctx));
-    if (n) { H2D(ctx, dp, points, 64 * n); H2D(ctx, ds, scalars, 32 * n); }
-    OG_TRY(msm_g1_dev(ctx, dp, ds, n, dout));
-    D2H(ctx, out64, dout, 64);
-    return check_flag(ctx);
+    return msm_host_entry<Fq>(ctx, points, scalars, n, out64);
 }
 int32_t og_msm_g2(og_ctx* ctx, const uint8_t* points, const uint8_t* scalars, uint64_t n, uint8_t* out128) {
-    OG_ENTER(ctx);
-    if (!ctx || !out128 || (n && (!points || !scalars))) return OG_E_INVALID;
-    OG_SLOT(ctx, dp, uint8_t, S_IO_A, 128 * n);
-    OG_SLOT(ctx, ds, uint8_t, S_IO_B, 32 * n);
-    OG_SLOT(ctx, dout, uint8_t, S_IO_C, 128);
-    OG_TRY(clear_flag(ctx));
-    if (n) { H2D(ctx, dp, points, 128 * n); H2D(ctx, ds, scalars, 32 * n); }
-    OG_TRY(msm_g2_dev(ctx, dp, ds, n, dout));
-    D2H(ctx, out128, dout, 128);
-    return check_flag(ctx);
+    return msm_host_entry<Fq2>(ctx, points, scalars, n, out128);
 }
-int32_t og_g1_sum(og_ctx* ctx, const uint8_t* points, uint64_t n, uint8_t* out64) {
-    OG_ENTER(ctx);
-    if (!ctx || !out64 || (n && !points)) return OG_E_INVALID;
-    OG_SLOT(ctx, dp, uint8_t, S_IO_A, 64 * n);
-    OG_SLOT(ctx, dout, uint8_t, S_IO_C, 64);
-    OG_TRY(clear_flag(ctx));
-    if (n) H2D(ctx, dp, points, 64 * n);
-    OG_TRY(sum_g1_dev(ctx, dp, n, dout));
-    D2H(ctx, out64, dout, 64);
-    return check_flag(ctx);
-}
-int32_t og_g2_sum(og_ctx* ctx, const uint8_t* points, uint64_t n, uint8_t* out128) {
-    OG_ENTER(ctx);
-    if (!ctx || !out128 || (n && !points)) return OG_E_INVALID;
-    OG_SLOT(ctx, dp, uint8_t, S_IO_A, 128 * n);
-    OG_SLOT(ctx, dout, uint8_t, S_IO_C, 128);
-    OG_TRY(clear_flag(ctx));
-    if (n) H2D(ctx, dp, points, 128 * n);
-    OG_TRY(sum_g2_dev(ctx, dp, n, dout));
-    D2H(ctx, out128, dout, 128);
-    return check_flag(ctx);
-}
+int32_t og_g1_sum(og_ctx* ctx, const uint8_t* points, uint64_t n, uint8_t* out64) { return sum_host_entry<Fq>(ctx, points, n, out64); }
+int32_t og_g2_sum(og_ctx* ctx, const uint8_t* points, uint64_t n, uint8_t* out128) { return sum_host_entry<Fq2>(ctx, points, n, out128); }
 
-int32_t og_g1_sum_dev(og_ctx* ctx, const uint8_t* d_points, uint64_t n, uint8_t* d_out64) {
-    OG_ENTER(ctx);
-    if (!d_out64 || (n && !d_points)) return OG_E_INVALID;
-    return sum_g1_dev(ctx, d_points, n, d_out64);
-}
-int32_t og_g2_sum_dev(og_ctx* ctx, const uint8_t* d_points, uint64_t n, uint8_t* d_out128) {
-    OG_ENTER(ctx);
-    if (!d_out128 || (n && !d_points)) return OG_E_INVALID;
-    return sum_g2_dev(ctx, d_points, n, d_out128);
-}
+int32_t og_g1_sum_dev(og_ctx* ctx, const uint8_t* d_points, uint64_t n, uint8_t* d_out64) { return sum_dev_entry<Fq>(ctx, d_points, n, d_out64); }
+int32_t og_g2_sum_dev(og_ctx* ctx, const uint8_t* d_points, uint64_t n, uint8_t* d_out128) { return sum_dev_entry<Fq2>(ctx, d_points, n, d_out128); }
 int32_t og_g1_generator_mul_dev(og_ctx* ctx, const uint8_t* d_scalars, uint64_t n, uint8_t* d_out_points) {
-    OG_ENTER(ctx);
-    if (n && (!d_scalars || !d_out_points)) return OG_E_INVALID;
-    if (n == 0) return OG_OK;
-    OG_SLOT(ctx, dp, G1Affine, S_IO_B, sizeof(G1Affine) * n);
-    OG_TRY(fixed_base_mul_g1(ctx, d_scalars, n, dp));
-    return g1_mont_to_bytes(ctx, dp, n, d_out_points);
+    return generator_mul_dev_entry<Fq>(ctx, d_scalars, n, d_out_points);
 }
 int32_t og_g2_generator_mul_dev(og_ctx* ctx, const uint8_t* d_scalars, uint64_t n, uint8_t* d_out_points) {
-    OG_ENTER(ctx);
-    if (n && (!d_scalars || !d_out_points)) return OG_E_INVALID;
-    if (n == 0) return OG_OK;
-    OG_SLOT(ctx, dp, G2Affine, S_IO_B, sizeof(G2Affine) * n);
-    OG_TRY(fixed_base_mul_g2(ctx, d_scalars, n, dp));
-    return g2_mont_to_bytes(ctx, dp, n, d_out_points);
+    return generator_mul_dev_entry<Fq2>(ctx, d_scalars, n, d_out_points);
 }
 
 // out[i] = scalars[i] * G (fixed-base, generator of G1 / G2): used by the setup and to synthesise MSM inputs
 int32_t og_g1_generator_mul(og_ctx* ctx, const uint8_t* scalars, uint64_t n, uint8_t* out_points) {
-    OG_ENTER(ctx);
-    if (!ctx || (n && (!scalars || !out_points))) return OG_E_INVALID;
-    if (n == 0) return OG_OK;
-    OG_SLOT(ctx, ds, uint8_t, S_IO_A, 32 * n);
-    OG_SLOT(ctx, dp, G1Affine, S_IO_B, sizeof(G1Affine) * n);
-    OG_SLOT(ctx, dout, uint8_t, S_IO_C, 64 * n);
-    OG_TRY(clear_flag(ctx));
-    H2D(ctx, ds, scalars, 32 * n);
-    OG_TRY(fixed_base_mul_g1(ctx, ds, n, dp));
-    OG_TRY(g1_mont_to_bytes(ctx, dp, n, dout));
-    D2H(ctx, out_points, dout, 64 * n);
-    return check_flag(ctx);
+    return generator_mul_host_entry<Fq>(ctx, scalars, n, out_points);
 }
 int32_t og_g2_generator_mul(og_ctx* ctx, const uint8_t* scalars, uint64_t n, uint8_t* out_points) {
-    OG_ENTER(ctx);
-    if (!ctx || (n && (!scalars || !out_points))) return OG_E_INVALID;
-    if (n == 0) return OG_OK;
-    OG_SLOT(ctx, ds, uint8_t, S_IO_A, 32 * n);
-    OG_SLOT(ctx, dp, G2Affine, S_IO_B, sizeof(G2Affine) * n);
-    OG_SLOT(ctx, dout, uint8_t, S_IO_C, 128 * n);
-    OG_TRY(clear_flag(ctx));
-    H2D(ctx, ds, scalars, 32 * n);
-    OG_TRY(fixed_base_mul_g2(ctx, ds, n, dp));
-    OG_TRY(g2_mont_to_bytes(ctx, dp, n, dout));
-    D2H(ctx, out_points, dout, 128 * n);
-    return check_flag(ctx);
+    return generator_mul_host_entry<Fq2>(ctx, scalars, n, out_points);
 }
 
 // ---- NTT ----------------------------------------------------------------------------------------------------

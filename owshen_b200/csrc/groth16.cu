@@ -228,6 +228,18 @@ void pk_free(og_pk* pk) {
     delete pk;
 }
 
+// stage a base-point list (boundary bytes), convert it to Montgomery form and extend it to the window table of MSM `which`
+template <class F>
+static int32_t load_table(og_ctx* ctx, const og_pk* pk, int which, const std::vector<uint8_t>& pts, uint32_t n, Affine<F>** table) {
+    uint8_t* stage;
+    OG_TRY(upload(ctx, &stage, pts.data(), pts.size()));
+    if (cudaMalloc(table, sizeof(Affine<F>) * (size_t)n * pk->n_windows[which]) != cudaSuccess) { cudaFree(stage); return OG_E_NOMEM; }
+    int32_t rc = points_to_mont(ctx, stage, n, *table);
+    if (rc == OG_OK) rc = build_table(ctx, *table, n, pk->c[which], pk->n_windows[which]);
+    cudaStreamSynchronize(ctx->stream); cudaFree(stage);
+    return rc;
+}
+
 int32_t pk_load(og_ctx* ctx, const uint8_t* bytes, uint64_t len, og_pk** out) {
     Reader rd{bytes, len};
     const uint8_t* magic = rd.take(4);
@@ -277,33 +289,9 @@ int32_t pk_load(og_ctx* ctx, const uint8_t* bytes, uint64_t len, og_pk** out) {
     int32_t rc = OG_OK;
     auto fail = [&](int32_t code) { pk_free(pk); return code; };
     if ((rc = clear_flag(ctx)) != OG_OK) return fail(rc);
-    {
-        uint8_t* stage;
-        if ((rc = upload(ctx, &stage, hA.data(), hA.size())) != OG_OK) return fail(rc);
-        if (cudaMalloc(&pk->tabA, sizeof(G1Affine) * (size_t)pk->nA * pk->n_windows[0]) != cudaSuccess) { cudaFree(stage); return fail(OG_E_NOMEM); }
-        rc = g1_bytes_to_mont(ctx, stage, pk->nA, pk->tabA);
-        if (rc == OG_OK) rc = msm_build_table_g1(ctx, pk->tabA, pk->nA, pk->c[0], pk->n_windows[0]);
-        cudaStreamSynchronize(ctx->stream); cudaFree(stage);
-        if (rc != OG_OK) return fail(rc);
-    }
-    {
-        uint8_t* stage;
-        if ((rc = upload(ctx, &stage, hC.data(), hC.size())) != OG_OK) return fail(rc);
-        if (cudaMalloc(&pk->tabC, sizeof(G1Affine) * (size_t)pk->nC * pk->n_windows[2]) != cudaSuccess) { cudaFree(stage); return fail(OG_E_NOMEM); }
-        rc = g1_bytes_to_mont(ctx, stage, pk->nC, pk->tabC);
-        if (rc == OG_OK) rc = msm_build_table_g1(ctx, pk->tabC, pk->nC, pk->c[2], pk->n_windows[2]);
-        cudaStreamSynchronize(ctx->stream); cudaFree(stage);
-        if (rc != OG_OK) return fail(rc);
-    }
-    {
-        uint8_t* stage;
-        if ((rc = upload(ctx, &stage, hB.data(), hB.size())) != OG_OK) return fail(rc);
-        if (cudaMalloc(&pk->tabB, sizeof(G2Affine) * (size_t)pk->nB * pk->n_windows[1]) != cudaSuccess) { cudaFree(stage); return fail(OG_E_NOMEM); }
-        rc = g2_bytes_to_mont(ctx, stage, pk->nB, pk->tabB);
-        if (rc == OG_OK) rc = msm_build_table_g2(ctx, pk->tabB, pk->nB, pk->c[1], pk->n_windows[1]);
-        cudaStreamSynchronize(ctx->stream); cudaFree(stage);
-        if (rc != OG_OK) return fail(rc);
-    }
+    if ((rc = load_table(ctx, pk, 0, hA, pk->nA, &pk->tabA)) != OG_OK) return fail(rc);
+    if ((rc = load_table(ctx, pk, 2, hC, pk->nC, &pk->tabC)) != OG_OK) return fail(rc);
+    if ((rc = load_table(ctx, pk, 1, hB, pk->nB, &pk->tabB)) != OG_OK) return fail(rc);
     if ((rc = upload(ctx, &pk->supp, supp.data(), 4ull * supp.size())) != OG_OK) return fail(rc);
     cudaStreamSynchronize(ctx->stream);
     if ((rc = upload_csr(ctx, rd, pk->n_constraints, nv, &pk->a_ptr, &pk->a_col, &pk->a_val)) != OG_OK) return fail(rc);
@@ -328,8 +316,9 @@ void pk_info(const og_pk* pk, uint32_t* n_vars, uint32_t* n_pub, uint32_t* log_m
 struct ChunkBufs {
     Fr *W, *rs_m, *abc, *ntt_tmp, *bsc, *csc;
     uint32_t *counts, *offsets, *cursor, *sorted, *heavy;
-    G1XYZZ *bk1, *lvl1, *totA, *totC;
-    G2XYZZ *bk2, *lvl2, *totB;
+    void *buckets, *lvl;                 // bucket and reduction scratch of one MSM (sized for G2; the MSMs run one after another)
+    G1XYZZ *totA, *totC;
+    G2XYZZ* totB;
     uint32_t w_stride, bsc_stride, csc_stride;
 };
 
@@ -350,22 +339,21 @@ static int32_t alloc_chunk(og_ctx* ctx, const og_pk* pk, uint32_t batch, uint32_
     b.offsets = (uint32_t*)ctx->slot(S_PR_OFFSETS, 4 * (n_keys + 1));
     b.cursor = (uint32_t*)ctx->slot(S_PR_CURSOR, 4 * n_keys);
     b.heavy = (uint32_t*)ctx->slot(S_PR_HEAVY, 4 * (2 * n_keys + 4));
-    b.bk2 = (G2XYZZ*)ctx->slot(S_PR_BUCKETS, sizeof(G2XYZZ) * n_keys);
-    b.lvl2 = (G2XYZZ*)ctx->slot(S_PR_SEG, sizeof(G2XYZZ) * msm_lvl_elems(B, pk->max_nb));
+    b.buckets = ctx->slot(S_PR_BUCKETS, sizeof(G2XYZZ) * n_keys);
+    b.lvl = ctx->slot(S_PR_SEG, sizeof(G2XYZZ) * msm_lvl_elems(B, pk->max_nb));
     b.totA = (G1XYZZ*)ctx->slot(S_PR_SUMS, (sizeof(G1XYZZ) * 2 + sizeof(G2XYZZ)) * (size_t)batch);
-    if (!b.W || !b.rs_m || !b.abc || !b.bsc || !b.sorted || !b.counts || !b.offsets || !b.cursor || !b.heavy || !b.bk2 || !b.lvl2 || !b.totA)
+    if (!b.W || !b.rs_m || !b.abc || !b.bsc || !b.sorted || !b.counts || !b.offsets || !b.cursor || !b.heavy || !b.buckets || !b.lvl || !b.totA)
         return OG_E_NOMEM;
     b.ntt_tmp = b.abc + (size_t)B * 3 * m;
     b.csc = b.bsc + (size_t)B * b.bsc_stride;
-    b.bk1 = reinterpret_cast<G1XYZZ*>(b.bk2);       // the G1 and G2 MSMs of a chunk run one after another
-    b.lvl1 = reinterpret_cast<G1XYZZ*>(b.lvl2);
     b.totC = b.totA + batch;
     b.totB = reinterpret_cast<G2XYZZ*>(b.totC + batch);
     return OG_OK;
 }
 
-static int32_t run_msm_g1(og_ctx* ctx, const og_pk* pk, int which, ChunkBufs& b, uint32_t B, const G1Affine* table, uint32_t n_pts,
-                          const Fr* scalars, uint32_t stride, G1XYZZ* totals) {
+template <class F>
+static int32_t run_msm(og_ctx* ctx, const og_pk* pk, int which, ChunkBufs& b, uint32_t B, const Affine<F>* table, uint32_t n_pts,
+                       const Fr* scalars, uint32_t stride, XYZZ<F>* totals) {
     DigitPlan plan;
     plan.scalars = reinterpret_cast<const uint32_t*>(scalars);
     plan.n = n_pts; plan.scalar_stride = stride; plan.n_problems = B;
@@ -374,19 +362,8 @@ static int32_t run_msm_g1(og_ctx* ctx, const og_pk* pk, int which, ChunkBufs& b,
     plan.montgomery = 1;
     uint32_t n_keys = B * pk->nb[which];
     OG_TRY(msm_sort_digits(ctx, plan, n_keys, b.counts, b.offsets, b.cursor, b.sorted));
-    return msm_buckets_g1(ctx, table, b.sorted, b.offsets, b.counts, B, pk->nb[which], (uint64_t)B * n_pts * pk->n_windows[which], b.bk1, b.lvl1, b.heavy, b.cursor, totals);
-}
-static int32_t run_msm_g2(og_ctx* ctx, const og_pk* pk, int which, ChunkBufs& b, uint32_t B, const G2Affine* table, uint32_t n_pts,
-                          const Fr* scalars, uint32_t stride, G2XYZZ* totals) {
-    DigitPlan plan;
-    plan.scalars = reinterpret_cast<const uint32_t*>(scalars);
-    plan.n = n_pts; plan.scalar_stride = stride; plan.n_problems = B;
-    plan.c = pk->c[which]; plan.n_windows = pk->n_windows[which]; plan.nb = pk->nb[which];
-    plan.key_stride_problem = 1; plan.key_stride_window = 0; plan.tidx_window_stride = n_pts;
-    plan.montgomery = 1;
-    uint32_t n_keys = B * pk->nb[which];
-    OG_TRY(msm_sort_digits(ctx, plan, n_keys, b.counts, b.offsets, b.cursor, b.sorted));
-    return msm_buckets_g2(ctx, table, b.sorted, b.offsets, b.counts, B, pk->nb[which], (uint64_t)B * n_pts * pk->n_windows[which], b.bk2, b.lvl2, b.heavy, b.cursor, totals);
+    return msm_buckets(ctx, table, b.sorted, b.offsets, b.counts, B, pk->nb[which], (uint64_t)B * n_pts * pk->n_windows[which],
+                       static_cast<XYZZ<F>*>(b.buckets), static_cast<XYZZ<F>*>(b.lvl), b.heavy, b.cursor, totals);
 }
 
 // where a chunk's witness rows come from
@@ -421,9 +398,9 @@ static int32_t prove_chunk(og_ctx* ctx, const og_pk* pk, ChunkBufs& b, const Wit
     OG_LAUNCH(ctx, k_compose, dim3((mx + 127) / 128, B), 128, 0, W, b.w_stride, rs_m, pk->supp, pk->n_supp, pk->n_vars, pk->n_pub, m,
               b.bsc, b.bsc_stride, b.csc, b.csc_stride);
     OG_LAUNCH(ctx, k_pointwise, dim3((m + 127) / 128, B), 128, 0, b.abc, pk->log_m, B, b.csc, b.csc_stride, n_priv + pk->n_supp);
-    OG_TRY(run_msm_g1(ctx, pk, 0, b, B, pk->tabA, pk->nA, W, b.w_stride, b.totA + off));
-    OG_TRY(run_msm_g1(ctx, pk, 2, b, B, pk->tabC, pk->nC, b.csc, b.csc_stride, b.totC + off));
-    OG_TRY(run_msm_g2(ctx, pk, 1, b, B, pk->tabB, pk->nB, b.bsc, b.bsc_stride, b.totB + off));
+    OG_TRY(run_msm(ctx, pk, 0, b, B, pk->tabA, pk->nA, W, b.w_stride, b.totA + off));
+    OG_TRY(run_msm(ctx, pk, 2, b, B, pk->tabC, pk->nC, b.csc, b.csc_stride, b.totC + off));
+    OG_TRY(run_msm(ctx, pk, 1, b, B, pk->tabB, pk->nB, b.bsc, b.bsc_stride, b.totB + off));
     OG_LAUNCH(ctx, k_assemble_g1, (B + 31) / 32, 32, 0, b.totA + off, b.totC + off, rs_m, B, d_proofs + 256ull * off);
     OG_LAUNCH(ctx, k_assemble_g2, (B + 31) / 32, 32, 0, b.totB + off, B, d_proofs + 256ull * off);
     return OG_OK;

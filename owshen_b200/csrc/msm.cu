@@ -2,21 +2,22 @@
 // for sm_100a.  BASELINE configs 3 and 5 and the inner engine of the batched Groth16 prover.
 //
 // No counterpart in the reference (SURVEY.md section 0).  Pipeline (DESIGN.md section 5.3):
-//   1. k_digits<false>   signed c-bit digits of every scalar, histogram of (group, bucket) keys
-//   2. k_scan            exclusive prefix sum of the histogram
-//   3. k_digits<true>    counting-sort scatter of (point index, sign) entries  -> coalesced bucket lists
-//   4. k_bucket_acc      one thread per bucket: XYZZ += affine point (8M+2S), accumulator in registers
-//      k_bucket_heavy    buckets above a cap get a whole CTA (witness-like scalars: 0/1 pile-ups)
-//   5. k_reduce_level    sum_b (b+1) B_b by 32-way running sums, log_32(nb) levels
-//   6. k_group_total / k_horner
-// All arithmetic is 8x32-bit Montgomery limbs in registers (fp.cuh); the kernels are bound by the
-// integer multiply-add pipe, not HBM: a G1 mixed add moves 64 B + 4 B and costs ~3.5k instructions.
+//   1-3. msm_sort.cu     signed c-bit digits -> histogram -> exclusive scan -> counting-sort scatter of
+//                        (point index, sign) entries: one coalesced list per bucket
+//   3b. k_bucket_order   bucket ids of every group ordered by decreasing load
+//   4. k_bucket_acc      one thread per bucket: XYZZ += affine point (8M+2S), accumulator in shared memory
+//      k_bucket_heavy    buckets above a cap are cut into segments of one CTA each (witness-like scalars: 0/1 pile-ups)
+//   5. k_reduce_level    sum_b (b+1) B_b by 8-way running sums, log_8(nb) levels; one-shot MSMs take the levels
+//                        above 0 as tree sums (k_tail_sums / k_tail_finish)
+//   6. k_group_total (prover) / k_horner over the windows (one-shot MSM)
+// All arithmetic is 8x32-bit Montgomery limbs (fp.cuh); the kernels are bound by the integer multiply-add pipe,
+// not HBM: a G1 mixed add moves 64 B + 4 B and costs ~3.5k instructions.
+//
+// Everything here is a template over the coordinate field F (Fq for G1, Fq2 for G2).  The file is compiled once per
+// field (-DOG_MSM_G1 / -DOG_MSM_G2, see the end of the file), so that the two heavy units build in parallel and the G2
+// unit can keep its Fq2 products out of line (-DOG_FP_MUL_CALL).
 #include "msm.cuh"
 #include "glv.cuh"
-// Compiled twice: -DOG_MSM_G1 (G1 instantiations + the curve-independent sort) and -DOG_MSM_G2.
-#if !defined(OG_MSM_G1) && !defined(OG_MSM_G2)
-#error "compile msm.cu with -DOG_MSM_G1 or -DOG_MSM_G2"
-#endif
 
 namespace og {
 
@@ -53,208 +54,16 @@ __global__ void __launch_bounds__(128) k_points_from_mont(const Affine<F>* __res
     FieldIO<F>::store(out + 2 * B * i + B, p.y);
 }
 
-#ifdef OG_MSM_G1
-int32_t g1_bytes_to_mont(og_ctx* ctx, const uint8_t* d_in, uint64_t n, G1Affine* d_out) {
-    if (n) OG_LAUNCH(ctx, k_points_to_mont<Fq>, (unsigned)((n + 127) / 128), 128, 0, d_in, n, d_out, ctx->d_flag);
+template <class F>
+int32_t points_to_mont(og_ctx* ctx, const uint8_t* d_in, uint64_t n, Affine<F>* d_out) {
+    if (n) OG_LAUNCH(ctx, k_points_to_mont<F>, (unsigned)((n + 127) / 128), 128, 0, d_in, n, d_out, ctx->d_flag);
     return OG_OK;
 }
-#endif  // OG_MSM_G1
-
-#ifdef OG_MSM_G2
-int32_t g2_bytes_to_mont(og_ctx* ctx, const uint8_t* d_in, uint64_t n, G2Affine* d_out) {
-    if (n) OG_LAUNCH(ctx, k_points_to_mont<Fq2>, (unsigned)((n + 127) / 128), 128, 0, d_in, n, d_out, ctx->d_flag);
+template <class F>
+int32_t points_to_bytes(og_ctx* ctx, const Affine<F>* d_in, uint64_t n, uint8_t* d_out) {
+    if (n) OG_LAUNCH(ctx, k_points_from_mont<F>, (unsigned)((n + 127) / 128), 128, 0, d_in, n, d_out);
     return OG_OK;
 }
-#endif  // OG_MSM_G2
-
-#ifdef OG_MSM_G1
-int32_t g1_mont_to_bytes(og_ctx* ctx, const G1Affine* d_in, uint64_t n, uint8_t* d_out) {
-    if (n) OG_LAUNCH(ctx, k_points_from_mont<Fq>, (unsigned)((n + 127) / 128), 128, 0, d_in, n, d_out);
-    return OG_OK;
-}
-#endif  // OG_MSM_G1
-
-#ifdef OG_MSM_G2
-int32_t g2_mont_to_bytes(og_ctx* ctx, const G2Affine* d_in, uint64_t n, uint8_t* d_out) {
-    if (n) OG_LAUNCH(ctx, k_points_from_mont<Fq2>, (unsigned)((n + 127) / 128), 128, 0, d_in, n, d_out);
-    return OG_OK;
-}
-#endif  // OG_MSM_G2
-
-
-#ifdef OG_MSM_G1
-// ---- 1/3: digits -> histogram / scatter ---------------------------------------------------------------
-// Signed c-bit digits of one scalar: v = bits + carry; v > 2^(c-1) -> digit v - 2^c, carry 1.  n_windows*c >= 255
-// guarantees that the top window absorbs the last carry for every scalar < r < 2^254.
-struct DigitIter {
-    uint32_t s[9];
-    __device__ __forceinline__ bool load(const DigitPlan& P, uint32_t prob, uint64_t i, int* flag) {
-        const uint32_t* sp = P.scalars + ((uint64_t)prob * P.scalar_stride + i) * 8;
-        if (P.montgomery) {
-            Fr v;
-#pragma unroll
-            for (int j = 0; j < 8; j++) v.l[j] = sp[j];
-            v.to_canonical(s);
-        } else {
-#pragma unroll
-            for (int j = 0; j < 8; j++) s[j] = sp[j];
-            if (!Fr::canonical_lt_mod(s)) { atomicOr(flag, 1); return false; }
-        }
-        s[8] = 0;
-        return (s[0] | s[1] | s[2] | s[3] | s[4] | s[5] | s[6] | s[7]) != 0;
-    }
-    // calls f(window, magnitude - 1, negative) for every non-zero signed digit
-    template <class Fn>
-    __device__ __forceinline__ void for_each(const DigitPlan& P, Fn f) const {
-        const uint32_t c = P.c, half = 1u << (c - 1), mask = (1u << c) - 1;
-        uint32_t carry = 0;
-        for (uint32_t w = 0; w < P.n_windows; w++) {
-            uint32_t bit = w * c, word = bit >> 5, sh = bit & 31;
-            uint64_t two = ((uint64_t)s[word + 1] << 32) | s[word];
-            uint32_t v = ((uint32_t)(two >> sh) & mask) + carry;
-            uint32_t neg = v > half;
-            uint32_t mag = neg ? (1u << c) - v : v;
-            carry = neg;
-            if (mag) f(w, mag - 1, neg);
-        }
-    }
-};
-
-// one thread per scalar, global atomics (one-shot MSMs: up to 2^15 buckets x 16 windows of keys).  The scatter is pure
-// atomic round-trip latency (ncu, profiles/r2_ncu_digits.md: 93 % of the warp samples on the long scoreboard, issue slots 17 %
-// busy); cutting eight windows first and issuing their eight atomics back to back was measured SLOWER (21.3 vs 20.1 ms per 1024
-// proofs, profiles/r2_small_ab.md): the L2 atomic units, not the per-thread dependency, are what the kernel waits for.
-template <bool SCATTER>
-__global__ void __launch_bounds__(256) k_digits(DigitPlan P, uint32_t* __restrict__ counts, const uint32_t* __restrict__ offsets,
-                                                uint32_t* __restrict__ cursor, uint32_t* __restrict__ sorted, int* flag) {
-    uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    uint32_t prob = blockIdx.y;
-    if (i >= P.n) return;
-    DigitIter it;
-    if (!it.load(P, prob, i, flag)) return;
-    it.for_each(P, [&](uint32_t w, uint32_t b, uint32_t neg) {
-        uint32_t key = (prob * P.key_stride_problem + w * P.key_stride_window) * P.nb + b;
-        if (!SCATTER) {
-            atomicAdd(&counts[key], 1u);
-        } else {
-            uint32_t pos = atomicAdd(&cursor[key], 1u);          // cursor starts at the bucket's offset (k_scan_apply)
-            sorted[pos] = (((uint32_t)i + w * P.tidx_window_stride) << 1) | neg;
-        }
-    });
-}
-
-// Tiled histogram for the batched prover (one group per proof, nb <= 32768): a CTA owns a tile of one problem's
-// scalars, counts its digits in shared memory and touches global memory once per bucket instead of once per
-// digit (5x faster than global atomics: 5 vs 24 ms per 1024 proofs).  The scatter stays the plain k_digits<true>:
-// a tiled scatter with run reservation and a one-CTA-per-proof shared-memory sort were both measured slower
-// (39 vs 33 ms and 56.6 vs 29 ms per 1024 proofs, profiles/r1_*; their code was removed in round 2).
-constexpr uint32_t DIG_TILE = 4096, DIG_THREADS = 256, DIG_MAX_NB_COUNT = 32768;
-
-__global__ void __launch_bounds__(DIG_THREADS) k_digits_count_tiled(DigitPlan P, uint32_t* __restrict__ counts, int* flag) {
-    extern __shared__ uint32_t hist[];                    // nb counters (dynamic: up to 128 KB)
-    const uint32_t prob = blockIdx.y, nb = P.nb;
-    const uint64_t lo = (uint64_t)blockIdx.x * DIG_TILE;
-    const uint64_t hi = lo + DIG_TILE < P.n ? lo + DIG_TILE : P.n;
-    const uint32_t key0 = prob * P.key_stride_problem * nb;          // key_stride_window == 0 in this mode
-    for (uint32_t b = threadIdx.x; b < nb; b += DIG_THREADS) hist[b] = 0;
-    __syncthreads();
-    for (uint64_t i = lo + threadIdx.x; i < hi; i += DIG_THREADS) {
-        DigitIter it;
-        if (it.load(P, prob, i, flag)) it.for_each(P, [&](uint32_t, uint32_t b, uint32_t) { atomicAdd(&hist[b], 1u); });
-    }
-    __syncthreads();
-    for (uint32_t b = threadIdx.x; b < nb; b += DIG_THREADS) if (hist[b]) atomicAdd(&counts[key0 + b], hist[b]);
-}
-
-// ---- 2: exclusive scan: tile sums -> scan of the tile sums (one CTA) -> tile rescan with offsets ----------
-constexpr uint32_t SCAN_THREADS = 256, SCAN_PER_THREAD = 8, SCAN_TILE = SCAN_THREADS * SCAN_PER_THREAD;
-
-__device__ __forceinline__ uint32_t block_exclusive_scan(uint32_t v, uint32_t* total) {   // 256 threads
-    __shared__ uint32_t warp_sums[SCAN_THREADS / 32];
-    __shared__ uint32_t block_total;
-    uint32_t lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    uint32_t inc = v;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) { uint32_t t = __shfl_up_sync(0xffffffffu, inc, d); if (lane >= (uint32_t)d) inc += t; }
-    if (lane == 31) warp_sums[wid] = inc;
-    __syncthreads();
-    if (wid == 0) {
-        uint32_t w = lane < SCAN_THREADS / 32 ? warp_sums[lane] : 0, winc = w;
-#pragma unroll
-        for (int d = 1; d < 8; d <<= 1) { uint32_t t = __shfl_up_sync(0xffffffffu, winc, d); if (lane >= (uint32_t)d) winc += t; }
-        if (lane < SCAN_THREADS / 32) warp_sums[lane] = winc - w;
-        if (lane == SCAN_THREADS / 32 - 1) block_total = winc;
-    }
-    __syncthreads();
-    uint32_t r = inc - v + warp_sums[wid];
-    *total = block_total;
-    __syncthreads();
-    return r;
-}
-
-__global__ void __launch_bounds__(SCAN_THREADS) k_scan_tiles(const uint32_t* __restrict__ counts, uint32_t n, uint32_t* __restrict__ tile_sums) {
-    uint32_t base = blockIdx.x * SCAN_TILE + threadIdx.x * SCAN_PER_THREAD, s = 0;
-#pragma unroll
-    for (uint32_t k = 0; k < SCAN_PER_THREAD; k++) if (base + k < n) s += counts[base + k];
-    uint32_t total;
-    block_exclusive_scan(s, &total);
-    if (threadIdx.x == 0) tile_sums[blockIdx.x] = total;
-}
-// in-place exclusive scan of up to SCAN_TILE * 64 tile sums by one CTA
-__global__ void __launch_bounds__(SCAN_THREADS) k_scan_tile_sums(uint32_t* __restrict__ tile_sums, uint32_t n_tiles, uint32_t* __restrict__ grand_total) {
-    uint32_t run = 0;
-    for (uint32_t base = 0; base < n_tiles; base += SCAN_THREADS) {
-        uint32_t i = base + threadIdx.x;
-        uint32_t v = i < n_tiles ? tile_sums[i] : 0, total;
-        uint32_t ex = block_exclusive_scan(v, &total);
-        if (i < n_tiles) tile_sums[i] = run + ex;
-        run += total;
-    }
-    if (threadIdx.x == 0) *grand_total = run;
-}
-__global__ void __launch_bounds__(SCAN_THREADS) k_scan_apply(const uint32_t* __restrict__ counts, uint32_t n, const uint32_t* __restrict__ tile_sums,
-                                                            uint32_t* __restrict__ offsets, uint32_t* __restrict__ cursor) {
-    uint32_t base = blockIdx.x * SCAN_TILE + threadIdx.x * SCAN_PER_THREAD;
-    uint32_t c[SCAN_PER_THREAD], s = 0;
-#pragma unroll
-    for (uint32_t k = 0; k < SCAN_PER_THREAD; k++) { c[k] = base + k < n ? counts[base + k] : 0; s += c[k]; }
-    uint32_t total;
-    uint32_t run = tile_sums[blockIdx.x] + block_exclusive_scan(s, &total);
-#pragma unroll
-    for (uint32_t k = 0; k < SCAN_PER_THREAD; k++) {      // the scatter's cursors start at the offsets: one random access per entry fewer
-        if (base + k < n) { offsets[base + k] = run; cursor[base + k] = run; }
-        run += c[k];
-    }
-}
-
-int32_t msm_sort_digits(og_ctx* ctx, const DigitPlan& plan, uint32_t n_keys, uint32_t* d_counts, uint32_t* d_offsets,
-                        uint32_t* d_cursor, uint32_t* d_sorted) {
-    OG_CUDA(ctx, cudaMemsetAsync(d_counts, 0, sizeof(uint32_t) * (size_t)n_keys, ctx->stream));
-    if (plan.n == 0 || plan.n_problems == 0) {
-        OG_CUDA(ctx, cudaMemsetAsync(d_offsets, 0, sizeof(uint32_t) * ((size_t)n_keys + 1), ctx->stream));
-        return OG_OK;
-    }
-    const bool tiled = plan.key_stride_window == 0 && plan.nb <= DIG_MAX_NB_COUNT;
-    if (tiled && !ctx->digits_smem_opt_in) {      // per device, hence per context
-        OG_CUDA(ctx, cudaFuncSetAttribute(k_digits_count_tiled, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(4 * DIG_MAX_NB_COUNT)));
-        ctx->digits_smem_opt_in = true;
-    }
-    dim3 grid((unsigned)((plan.n + 255) / 256), plan.n_problems);
-    dim3 tgrid((unsigned)((plan.n + DIG_TILE - 1) / DIG_TILE), plan.n_problems);
-    if (tiled) OG_LAUNCH(ctx, k_digits_count_tiled, tgrid, DIG_THREADS, 4 * (size_t)plan.nb, plan, d_counts, ctx->d_flag);
-    else OG_LAUNCHN(ctx, "k_digits_count", k_digits<false>, grid, 256, 0, plan, d_counts, nullptr, nullptr, nullptr, ctx->d_flag);
-    {   // offsets[n_keys] receives the grand total; cursor[k] = offsets[k] for the scatter
-        uint32_t n_tiles = (n_keys + SCAN_TILE - 1) / SCAN_TILE;
-        OG_SLOT(ctx, tile_sums, uint32_t, S_MSM_MISC, 4 * (size_t)n_tiles);
-        OG_LAUNCH(ctx, k_scan_tiles, n_tiles, SCAN_THREADS, 0, d_counts, n_keys, tile_sums);
-        OG_LAUNCH(ctx, k_scan_tile_sums, 1, SCAN_THREADS, 0, tile_sums, n_tiles, d_offsets + n_keys);
-        OG_LAUNCH(ctx, k_scan_apply, n_tiles, SCAN_THREADS, 0, d_counts, n_keys, tile_sums, d_offsets, d_cursor);
-    }
-    OG_LAUNCHN(ctx, "k_digits_scatter", k_digits<true>, grid, 256, 0, plan, d_counts, d_offsets, d_cursor, d_sorted, ctx->d_flag);
-    return OG_OK;
-}
-#endif  // OG_MSM_G1
-
 
 // ---- 3b: order the buckets of every group by decreasing load ------------------------------------------------
 // Bucket loads are Poisson-distributed, so a warp of 32 neighbouring buckets waits for its longest list
@@ -299,100 +108,75 @@ __device__ __forceinline__ Affine<F> fetch_point(const Affine<F>* __restrict__ t
     return p;
 }
 
-#ifdef OG_MSM_G1
-// G1 variant with the 128-byte accumulator in shared memory (see the G2 one below): 8 chunks of 16 bytes per thread.
-struct SmAcc1 {
-    uint4* base;    // [8 chunks][128 threads]
-    __device__ __forceinline__ Fq ld(int coord) const {
-        Fq v;
-        uint4 a = base[(coord * 2 + 0) * 128], b = base[(coord * 2 + 1) * 128];
-        v.l[0] = a.x; v.l[1] = a.y; v.l[2] = a.z; v.l[3] = a.w; v.l[4] = b.x; v.l[5] = b.y; v.l[6] = b.z; v.l[7] = b.w;
+// The accumulator lives in shared memory, 16-byte chunks interleaved over the CTA's 128 threads so that every access is
+// conflict-free (the layout of RedSm below): registers hold only the temporaries of one mixed addition, which buys resident
+// warps in a kernel whose top stall is the fixed-latency wait of the carry chains (profiles/r1_bucket_acc_smem_sweep.md).
+template <class F> struct SmAcc {
+    static constexpr int CH = sizeof(F) / 16;
+    uint4* base;    // [4 coordinates][CH chunks][128 threads]
+    // the Fq halves of a coordinate: the coordinate itself in G1, c0 and c1 in G2.  Limbs are copied one by one with constant
+    // indices: a reinterpret_cast of the coordinate, or a limb pointer, costs the G1 kernel 16 bytes of stack and 16 instructions.
+    static __device__ __forceinline__ Fq& half(Fq& v, int) { return v; }
+    static __device__ __forceinline__ const Fq& half(const Fq& v, int) { return v; }
+    static __device__ __forceinline__ Fq& half(Fq2& v, int h) { return h ? v.c1 : v.c0; }
+    static __device__ __forceinline__ const Fq& half(const Fq2& v, int h) { return h ? v.c1 : v.c0; }
+    __device__ __forceinline__ F ld(int coord) const {
+        uint4 q[CH];
+#pragma unroll
+        for (int c = 0; c < CH; c++) q[c] = base[(coord * CH + c) * 128];
+        F v;
+#pragma unroll
+        for (int c = 0; c < CH; c++) {
+            uint32_t* l = half(v, c >> 1).l + 4 * (c & 1);
+            l[0] = q[c].x; l[1] = q[c].y; l[2] = q[c].z; l[3] = q[c].w;
+        }
         return v;
     }
-    __device__ __forceinline__ void st(int coord, const Fq& v) const {
-        base[(coord * 2 + 0) * 128] = make_uint4(v.l[0], v.l[1], v.l[2], v.l[3]);
-        base[(coord * 2 + 1) * 128] = make_uint4(v.l[4], v.l[5], v.l[6], v.l[7]);
+    __device__ __forceinline__ void st(int coord, const F& v) const {
+#pragma unroll
+        for (int h = 0; h < CH / 2; h++) {
+            const Fq& x = half(v, h);
+            base[(coord * CH + 2 * h) * 128] = make_uint4(x.l[0], x.l[1], x.l[2], x.l[3]);
+            base[(coord * CH + 2 * h + 1) * 128] = make_uint4(x.l[4], x.l[5], x.l[6], x.l[7]);
+        }
     }
 };
 
-// 8 CTAs of 128 threads per SM (64 registers); only the next 4-byte ENTRY is read ahead, the 64-byte gather is
-// covered by the other warps (measured against 6/7 CTAs and against a prefetched point: profiles/r1_bucket_acc_smem_sweep.md)
-// the two squarings of a mixed addition through ONE out-of-line copy of the wide squarer (8 registers in, 8 out): with the squarer
-// inlined twice next to eight inlined products the kernel outgrew the instruction cache (ncu: 12.7 % of the warp samples waiting
-// for instructions after the wide squarer replaced the interleaved one, profiles/r2_small_ab.md)
+// What the bucket kernel does differently per field.
+template <class F> struct BucketAcc;
+// G1: 8 CTAs of 128 threads per SM (64 registers); only the next 4-byte ENTRY is read ahead, the 64-byte gather is covered by
+// the other warps (measured against 6/7 CTAs and against a prefetched point: profiles/r1_bucket_acc_smem_sweep.md).
+// The two squarings of a mixed addition go through ONE out-of-line copy of the wide squarer (8 registers in, 8 out): with the
+// squarer inlined twice next to eight inlined products the kernel outgrew the instruction cache (ncu: 12.7 % of the warp samples
+// waiting for instructions after the wide squarer replaced the interleaved one, profiles/r2_small_ab.md).
 static __device__ __noinline__ Fq fq_sqr_call(Fq a) { return a.sqr(); }
-__global__ void __launch_bounds__(128, 8) k_bucket_acc_sm1(const Affine<Fq>* __restrict__ table, const uint32_t* __restrict__ sorted,
-                                                        const uint32_t* __restrict__ offsets, const uint32_t* __restrict__ counts,
-                                                        uint32_t n_keys, uint32_t cap, XYZZ<Fq>* __restrict__ buckets,
-                                                        uint32_t* __restrict__ heavy, const uint32_t* __restrict__ perm) {
-    __shared__ uint4 sm_acc[8 * 128];
-    uint32_t slot_ = blockIdx.x * blockDim.x + threadIdx.x;
-    if (slot_ >= n_keys) return;
-    uint32_t key = perm[slot_];
-    uint32_t cnt = counts[key], off = offsets[key];
-    if (cnt > cap) {                               // left to k_bucket_heavy
-        uint32_t slot = atomicAdd(heavy, 1u);
-        heavy[1 + slot] = key;
-        buckets[key] = XYZZ<Fq>::inf();
-        return;
+template <> struct BucketAcc<Fq> {
+    static constexpr int MIN_CTAS = 8;
+    static __device__ __forceinline__ Fq sqr(const Fq& a) { return fq_sqr_call(a); }
+    // y3 = r (q1 - x3) - y ppp in the statement order each kernel was measured with: one order for both fields changes the
+    // other field's code (G1 with G2's order: 4160 -> 4152 SASS instructions; G2 with G1's: 3112 -> 3080), and neither
+    // alternative has been timed.
+    static __device__ __forceinline__ Fq y3(const SmAcc<Fq>& A, const Fq& r, const Fq& q1, const Fq& x3, const Fq& ppp) {
+        return r * (q1 - x3) - A.ld(1) * ppp;
     }
-    SmAcc1 A{sm_acc + threadIdx.x};
-    bool inf = true;
-    uint32_t e = cnt ? sorted[off] : 0;
-    for (uint32_t k = 0; k < cnt; k++) {
-        uint32_t en = k + 1 < cnt ? sorted[off + k + 1] : 0;
-        Affine<Fq> q = fetch_point(table, e);
-        e = en;
-        if (q.is_inf()) continue;
-        if (inf) { A.st(0, q.x); A.st(1, q.y); A.st(2, Fq::one()); A.st(3, Fq::one()); inf = false; continue; }
-        Fq p = q.x * A.ld(2) - A.ld(0);
-        Fq r = q.y * A.ld(3) - A.ld(1);
-        if (p.is_zero()) {
-            if (r.is_zero()) { XYZZ<Fq> d = XYZZ<Fq>::dbl_affine(q); A.st(0, d.x); A.st(1, d.y); A.st(2, d.zz); A.st(3, d.zzz); }
-            else inf = true;
-            continue;
-        }
-        // ordered so that few temporaries are live at a time: zz and zzz are updated as soon as pp / ppp exist
-        Fq pp = fq_sqr_call(p);
-        A.st(2, A.ld(2) * pp);
-        Fq ppp = p * pp;
-        A.st(3, A.ld(3) * ppp);
-        Fq q1 = A.ld(0) * pp;
-        Fq x3 = fq_sqr_call(r) - ppp - q1.dbl();
-        A.st(0, x3);
-        A.st(1, r * (q1 - x3) - A.ld(1) * ppp);
-    }
-    buckets[key] = inf ? XYZZ<Fq>::inf() : XYZZ<Fq>{A.ld(0), A.ld(1), A.ld(2), A.ld(3)};
-}
-#endif
-
-#ifdef OG_MSM_G2
-// G2 variant with the 256-byte accumulator in shared memory (16-byte chunks interleaved over the CTA's threads, so
-// every access is conflict-free): registers hold only the temporaries of one mixed addition, which buys resident
-// warps in a kernel whose top stall is the fixed-latency wait of the carry chains (4, 5 and 6 resident CTAs were measured
-// in round 1, profiles/r1_bucket_acc_smem_sweep.md; 6 won).
-struct SmAcc {
-    uint4* base;    // [16 chunks][128 threads]
-    __device__ __forceinline__ Fq2 ld(int coord) const {
-        Fq2 v;
-        uint4 a = base[(coord * 4 + 0) * 128], b = base[(coord * 4 + 1) * 128], c = base[(coord * 4 + 2) * 128], d = base[(coord * 4 + 3) * 128];
-        v.c0.l[0] = a.x; v.c0.l[1] = a.y; v.c0.l[2] = a.z; v.c0.l[3] = a.w; v.c0.l[4] = b.x; v.c0.l[5] = b.y; v.c0.l[6] = b.z; v.c0.l[7] = b.w;
-        v.c1.l[0] = c.x; v.c1.l[1] = c.y; v.c1.l[2] = c.z; v.c1.l[3] = c.w; v.c1.l[4] = d.x; v.c1.l[5] = d.y; v.c1.l[6] = d.z; v.c1.l[7] = d.w;
-        return v;
-    }
-    __device__ __forceinline__ void st(int coord, const Fq2& v) const {
-        base[(coord * 4 + 0) * 128] = make_uint4(v.c0.l[0], v.c0.l[1], v.c0.l[2], v.c0.l[3]);
-        base[(coord * 4 + 1) * 128] = make_uint4(v.c0.l[4], v.c0.l[5], v.c0.l[6], v.c0.l[7]);
-        base[(coord * 4 + 2) * 128] = make_uint4(v.c1.l[0], v.c1.l[1], v.c1.l[2], v.c1.l[3]);
-        base[(coord * 4 + 3) * 128] = make_uint4(v.c1.l[4], v.c1.l[5], v.c1.l[6], v.c1.l[7]);
+};
+// G2: 6 CTAs (4, 5 and 6 resident CTAs were measured in round 1, profiles/r1_bucket_acc_smem_sweep.md); Fq2 products and
+// squarings are out of line in this translation unit already (-DOG_FP_MUL_CALL, fp.cuh).
+template <> struct BucketAcc<Fq2> {
+    static constexpr int MIN_CTAS = 6;
+    static __device__ __forceinline__ Fq2 sqr(const Fq2& a) { return a.sqr(); }
+    static __device__ __forceinline__ Fq2 y3(const SmAcc<Fq2>& A, const Fq2& r, const Fq2& q1, const Fq2& x3, const Fq2& ppp) {
+        Fq2 t = A.ld(1) * ppp;
+        return r * (q1 - x3) - t;
     }
 };
 
-__global__ void __launch_bounds__(128, 6) k_bucket_acc_sm(const Affine<Fq2>* __restrict__ table, const uint32_t* __restrict__ sorted,
-                                                       const uint32_t* __restrict__ offsets, const uint32_t* __restrict__ counts,
-                                                       uint32_t n_keys, uint32_t cap, XYZZ<Fq2>* __restrict__ buckets,
-                                                       uint32_t* __restrict__ heavy, const uint32_t* __restrict__ perm) {
-    __shared__ uint4 sm_acc[16 * 128];
+template <class F>
+__global__ void __launch_bounds__(128, BucketAcc<F>::MIN_CTAS) k_bucket_acc(const Affine<F>* __restrict__ table, const uint32_t* __restrict__ sorted,
+                                                                           const uint32_t* __restrict__ offsets, const uint32_t* __restrict__ counts,
+                                                                           uint32_t n_keys, uint32_t cap, XYZZ<F>* __restrict__ buckets,
+                                                                           uint32_t* __restrict__ heavy, const uint32_t* __restrict__ perm) {
+    __shared__ uint4 sm_acc[4 * SmAcc<F>::CH * 128];
     uint32_t slot_ = blockIdx.x * blockDim.x + threadIdx.x;
     if (slot_ >= n_keys) return;
     uint32_t key = perm[slot_];
@@ -400,40 +184,38 @@ __global__ void __launch_bounds__(128, 6) k_bucket_acc_sm(const Affine<Fq2>* __r
     if (cnt > cap) {                               // left to k_bucket_heavy
         uint32_t slot = atomicAdd(heavy, 1u);
         heavy[1 + slot] = key;
-        buckets[key] = XYZZ<Fq2>::inf();
+        buckets[key] = XYZZ<F>::inf();
         return;
     }
-    SmAcc A{sm_acc + threadIdx.x};
+    SmAcc<F> A{sm_acc + threadIdx.x};
     bool inf = true;
     uint32_t e = cnt ? sorted[off] : 0;
     for (uint32_t k = 0; k < cnt; k++) {
         uint32_t en = k + 1 < cnt ? sorted[off + k + 1] : 0;
-        Affine<Fq2> q = fetch_point(table, e);
+        Affine<F> q = fetch_point(table, e);
         e = en;
         if (q.is_inf()) continue;
-        if (inf) { A.st(0, q.x); A.st(1, q.y); A.st(2, Fq2::one()); A.st(3, Fq2::one()); inf = false; continue; }
-        Fq2 p = q.x * A.ld(2) - A.ld(0);
-        Fq2 r = q.y * A.ld(3) - A.ld(1);
+        if (inf) { A.st(0, q.x); A.st(1, q.y); A.st(2, F::one()); A.st(3, F::one()); inf = false; continue; }
+        F p = q.x * A.ld(2) - A.ld(0);
+        F r = q.y * A.ld(3) - A.ld(1);
         if (p.is_zero()) {
-            if (r.is_zero()) { XYZZ<Fq2> d = XYZZ<Fq2>::dbl_affine(q); A.st(0, d.x); A.st(1, d.y); A.st(2, d.zz); A.st(3, d.zzz); }
+            if (r.is_zero()) { XYZZ<F> d = XYZZ<F>::dbl_affine(q); A.st(0, d.x); A.st(1, d.y); A.st(2, d.zz); A.st(3, d.zzz); }
             else inf = true;
             continue;
         }
-        // ordered so that few Fq2 temporaries are live across the out-of-line multiplier calls (each one is 16 registers
-        // that would otherwise be spilled around every call): zz and zzz are updated as soon as pp / ppp exist
-        Fq2 pp = p.sqr();
+        // ordered so that few temporaries are live at a time (in G2, across the out-of-line multiplier calls, each Fq2 one
+        // is 16 registers that would otherwise be spilled around every call): zz and zzz are updated as soon as pp / ppp exist
+        F pp = BucketAcc<F>::sqr(p);
         A.st(2, A.ld(2) * pp);
-        Fq2 ppp = p * pp;
+        F ppp = p * pp;
         A.st(3, A.ld(3) * ppp);
-        Fq2 q1 = A.ld(0) * pp;
-        Fq2 x3 = r.sqr() - ppp - q1.dbl();
+        F q1 = A.ld(0) * pp;
+        F x3 = BucketAcc<F>::sqr(r) - ppp - q1.dbl();
         A.st(0, x3);
-        Fq2 t = A.ld(1) * ppp;
-        A.st(1, r * (q1 - x3) - t);
+        A.st(1, BucketAcc<F>::y3(A, r, q1, x3, ppp));
     }
-    buckets[key] = inf ? XYZZ<Fq2>::inf() : XYZZ<Fq2>{A.ld(0), A.ld(1), A.ld(2), A.ld(3)};
+    buckets[key] = inf ? XYZZ<F>::inf() : XYZZ<F>{A.ld(0), A.ld(1), A.ld(2), A.ld(3)};
 }
-#endif
 
 // Heavy buckets (lists above the cap: witness-like scalars put 30 % of all points into bucket "1" of window 0) are cut
 // into segments of `seg` entries; every segment gets a CTA, a second kernel adds the partial sums of each bucket.
@@ -534,14 +316,12 @@ template <class F> struct RedOps {
     static __device__ __forceinline__ void add(XYZZ<F>& a, const XYZZ<F>& b) { a.add(b); }
     static __device__ __forceinline__ void dbl(XYZZ<F>& a) { a = a.dbl(); }
 };
-#ifdef OG_MSM_G1
 static __device__ __noinline__ XYZZ<Fq> g1_add_rv(XYZZ<Fq> a, XYZZ<Fq> b) { a.add(b); return a; }
 static __device__ __noinline__ XYZZ<Fq> g1_dbl_rv(XYZZ<Fq> a) { return a.dbl(); }
 template <> struct RedOps<Fq> {
     static __device__ __forceinline__ void add(XYZZ<Fq>& a, const XYZZ<Fq>& b) { a = g1_add_rv(a, b); }
     static __device__ __forceinline__ void dbl(XYZZ<Fq>& a) { a = g1_dbl_rv(a); }
 };
-#endif
 
 // measured (profiles/r2_small_ab.md): G1 25.5 (registers, out-of-line ops) vs 29.6 ms (shared memory); G2 25.3 (registers, spilling) vs 24.1 ms
 template <class F> constexpr bool RED_SM_DEFAULT = sizeof(F) != 32;
@@ -736,9 +516,9 @@ __global__ void __launch_bounds__(TAIL_THREADS) k_tail_finish(const XYZZ<F>* __r
 }
 
 template <class F>
-static int32_t msm_buckets(og_ctx* ctx, const Affine<F>* d_table, const uint32_t* d_sorted, const uint32_t* d_offsets,
+int32_t msm_buckets(og_ctx* ctx, const Affine<F>* d_table, const uint32_t* d_sorted, const uint32_t* d_offsets,
                            const uint32_t* d_counts, uint32_t n_groups, uint32_t nb, uint64_t n_entries_max, XYZZ<F>* d_buckets,
-                           XYZZ<F>* d_lvl, uint32_t* d_heavy, uint32_t* d_perm, XYZZ<F>* d_totals, bool few_groups = false) {
+                           XYZZ<F>* d_lvl, uint32_t* d_heavy, uint32_t* d_perm, XYZZ<F>* d_totals, bool few_groups) {
     uint32_t n_keys = n_groups * nb;
     constexpr int HT = sizeof(F) == 32 ? 256 : 128;
     OG_CUDA(ctx, cudaMemsetAsync(d_heavy, 0, sizeof(uint32_t), ctx->stream));
@@ -747,11 +527,8 @@ static int32_t msm_buckets(og_ctx* ctx, const Affine<F>* d_table, const uint32_t
     // (skewed scalars: witness 0/1 values, short scalars whose top window has few distinct digits)
     uint64_t avg = n_entries_max / (n_keys ? n_keys : 1);
     uint32_t cap = (uint32_t)(4 * avg < 128 ? 128 : 4 * avg);
-#ifdef OG_MSM_G1
-    OG_LAUNCHN(ctx, "k_bucket_acc_g1", k_bucket_acc_sm1, (n_keys + 127) / 128, 128, 0, d_table, d_sorted, d_offsets, d_counts, n_keys, cap, d_buckets, d_heavy, d_perm);
-#else
-    OG_LAUNCHN(ctx, "k_bucket_acc_g2", k_bucket_acc_sm, (n_keys + 127) / 128, 128, 0, d_table, d_sorted, d_offsets, d_counts, n_keys, cap, d_buckets, d_heavy, d_perm);
-#endif
+    OG_LAUNCHN(ctx, sizeof(F) == 32 ? "k_bucket_acc_g1" : "k_bucket_acc_g2", k_bucket_acc<F>, (n_keys + 127) / 128, 128, 0, d_table, d_sorted,
+               d_offsets, d_counts, n_keys, cap, d_buckets, d_heavy, d_perm);
     {
         // segment length: long enough that the segment sums of ALL heavy buckets fit in the (still unused) reduction scratch
         // (at most n_keys / 4 heavy buckets, since each holds more than 4 x the average load)
@@ -806,21 +583,6 @@ static int32_t msm_buckets(og_ctx* ctx, const Affine<F>* d_table, const uint32_t
     return OG_OK;
 }
 
-#ifdef OG_MSM_G1
-int32_t msm_buckets_g1(og_ctx* ctx, const G1Affine* d_table, const uint32_t* d_sorted, const uint32_t* d_offsets,
-                       const uint32_t* d_counts, uint32_t n_groups, uint32_t nb, uint64_t n_entries_max, G1XYZZ* d_buckets,
-                       G1XYZZ* d_lvl, uint32_t* d_heavy, uint32_t* d_perm, G1XYZZ* d_totals) {
-    return msm_buckets<Fq>(ctx, d_table, d_sorted, d_offsets, d_counts, n_groups, nb, n_entries_max, d_buckets, d_lvl, d_heavy, d_perm, d_totals);
-}
-#endif  // OG_MSM_G1
-
-#ifdef OG_MSM_G2
-int32_t msm_buckets_g2(og_ctx* ctx, const G2Affine* d_table, const uint32_t* d_sorted, const uint32_t* d_offsets,
-                       const uint32_t* d_counts, uint32_t n_groups, uint32_t nb, uint64_t n_entries_max, G2XYZZ* d_buckets,
-                       G2XYZZ* d_lvl, uint32_t* d_heavy, uint32_t* d_perm, G2XYZZ* d_totals) {
-    return msm_buckets<Fq2>(ctx, d_table, d_sorted, d_offsets, d_counts, n_groups, nb, n_entries_max, d_buckets, d_lvl, d_heavy, d_perm, d_totals);
-}
-#endif  // OG_MSM_G2
 
 
 // ---- 6: one-shot MSM = Horner over the window totals ------------------------------------------------------
@@ -890,11 +652,15 @@ __global__ void __launch_bounds__(128) k_horner(const XYZZ<F>* __restrict__ tota
     }
 }
 
+// GLV front end of the one-shot MSM (glv.cuh): only G1 has the endomorphism, so for any other field it does nothing.
+// G1: (P_i, k_i) -> (+-P_i, |k1_i|) at index i and (+-phi(P_i), |k2_i|) at index n + i; the signs go into the points and
+// d_scalars is pointed at the new scalars.  phi(P_i) is MATERIALISED: applying beta at fetch time instead (entries >= n standing
+// for phi of point index - n, signs in the scalars) keeps the table at 64 MB but costs a product per phi entry in the accumulation
+// kernel and measured 3.61 vs 3.27 ms of accumulation at 2^20 points (profiles/r2_msm_oneshot_breakdown.md)
+template <class F>
+static int32_t glv_expand(og_ctx*, const uint8_t*&, uint64_t, Affine<F>*) { return OG_OK; }
+
 #ifdef OG_MSM_G1
-// GLV front end of the one-shot G1 MSM (glv.cuh): (P_i, k_i) -> (+-P_i, |k1_i|) at index i and (+-phi(P_i), |k2_i|) at index n + i;
-// the signs go into the points.  phi(P_i) is MATERIALISED: applying beta at fetch time instead (entries >= n standing for phi of
-// point index - n, signs in the scalars) keeps the table at 64 MB but costs a product per phi entry in the accumulation kernel and
-// measured 3.61 vs 3.27 ms of accumulation at 2^20 points (profiles/r2_msm_oneshot_breakdown.md)
 __global__ void __launch_bounds__(128) k_glv_expand(const uint8_t* __restrict__ scalars, uint64_t n, Fq beta, Affine<Fq>* __restrict__ pts,
                                                     uint32_t* __restrict__ sc2, int* flag) {
     uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -921,7 +687,17 @@ __global__ void __launch_bounds__(128) k_glv_expand(const uint8_t* __restrict__ 
 #pragma unroll
     for (int j = 0; j < 8; j++) { o1[j] = m1[j]; o2[j] = m2[j]; }
 }
-#endif
+template <>
+int32_t glv_expand<Fq>(og_ctx* ctx, const uint8_t*& d_scalars, uint64_t n, Affine<Fq>* pts) {
+    OG_SLOT(ctx, sc2, uint32_t, S_MSM_SCALARS, 32 * 2 * (size_t)n);
+    uint32_t bl[8];
+    for (int i = 0; i < 8; i++) bl[i] = Glv::beta(i);
+    const Fq beta = Fq::from_canonical(bl);
+    OG_LAUNCH(ctx, k_glv_expand, (unsigned)((n + 127) / 128), 128, 0, d_scalars, n, beta, pts, sc2, ctx->d_flag);
+    d_scalars = reinterpret_cast<const uint8_t*>(sc2);
+    return OG_OK;
+}
+#endif  // OG_MSM_G1
 
 static uint32_t pick_window(uint64_t n) {
     uint32_t lg = 0;
@@ -933,7 +709,7 @@ static uint32_t pick_window(uint64_t n) {
 }
 
 template <class F>
-static int32_t msm_dev(og_ctx* ctx, const uint8_t* d_points, const uint8_t* d_scalars, uint64_t n, uint8_t* d_out) {
+int32_t msm_dev(og_ctx* ctx, const uint8_t* d_points, const uint8_t* d_scalars, uint64_t n, uint8_t* d_out) {
     constexpr int PB = 2 * FieldIO<F>::BYTES;
     if (n >= (1ull << 28)) return OG_E_INVALID;
     if (!aligned32(d_points) || !aligned32(d_scalars)) return OG_E_INVALID;
@@ -954,17 +730,8 @@ static int32_t msm_dev(og_ctx* ctx, const uint8_t* d_points, const uint8_t* d_sc
     OG_SLOT(ctx, lvl, XYZZ<F>, S_MSM_SEG, sizeof(XYZZ<F>) * msm_lvl_elems(W, nb));
     OG_SLOT(ctx, heavy, uint32_t, S_MSM_HEAVY, 4 * (2 * (size_t)n_keys + 4));
     OG_SLOT(ctx, totals, XYZZ<F>, S_MSM_OUT, sizeof(XYZZ<F>) * W);
-    OG_LAUNCH(ctx, k_points_to_mont<F>, (unsigned)((n_in + 127) / 128), 128, 0, d_points, n_in, pts, ctx->d_flag);
-#ifdef OG_MSM_G1
-    if (glv) {
-        OG_SLOT(ctx, sc2, uint32_t, S_MSM_SCALARS, 32 * (size_t)n);
-        uint32_t bl[8];
-        for (int i = 0; i < 8; i++) bl[i] = Glv::beta(i);
-        const Fq beta = Fq::from_canonical(bl);
-        OG_LAUNCH(ctx, k_glv_expand, (unsigned)((n_in + 127) / 128), 128, 0, d_scalars, n_in, beta, reinterpret_cast<Affine<Fq>*>(pts), sc2, ctx->d_flag);
-        d_scalars = reinterpret_cast<const uint8_t*>(sc2);
-    }
-#endif
+    OG_TRY(points_to_mont(ctx, d_points, n_in, pts));
+    if (glv) OG_TRY(glv_expand(ctx, d_scalars, n_in, pts));
     DigitPlan plan;
     plan.scalars = reinterpret_cast<const uint32_t*>(d_scalars);
     plan.n = n; plan.scalar_stride = 0; plan.n_problems = 1;
@@ -976,19 +743,6 @@ static int32_t msm_dev(og_ctx* ctx, const uint8_t* d_points, const uint8_t* d_sc
     OG_LAUNCH(ctx, k_horner<F>, 1, 128, 0, totals, W, c, d_out);
     return OG_OK;
 }
-
-#ifdef OG_MSM_G1
-int32_t msm_g1_dev(og_ctx* ctx, const uint8_t* d_points, const uint8_t* d_scalars, uint64_t n, uint8_t* d_out64) {
-    return msm_dev<Fq>(ctx, d_points, d_scalars, n, d_out64);
-}
-#endif  // OG_MSM_G1
-
-#ifdef OG_MSM_G2
-int32_t msm_g2_dev(og_ctx* ctx, const uint8_t* d_points, const uint8_t* d_scalars, uint64_t n, uint8_t* d_out128) {
-    return msm_dev<Fq2>(ctx, d_points, d_scalars, n, d_out128);
-}
-#endif  // OG_MSM_G2
-
 
 // ---- plain sum of affine points (post all-gather combine in the sharded MSM) ------------------------------------
 template <class F, int THREADS>
@@ -1015,22 +769,12 @@ __global__ void __launch_bounds__(THREADS) k_sum_points(const uint8_t* __restric
         FieldIO<F>::store(out + B, a.y);
     }
 }
-#ifdef OG_MSM_G1
-int32_t sum_g1_dev(og_ctx* ctx, const uint8_t* d_points, uint64_t n, uint8_t* d_out64) {
-    auto k = k_sum_points<Fq, 128>;
-    OG_LAUNCH(ctx, k, 1, 128, 128 * sizeof(G1XYZZ), d_points, n, d_out64, ctx->d_flag);
+template <class F>
+int32_t sum_points_dev(og_ctx* ctx, const uint8_t* d_points, uint64_t n, uint8_t* d_out) {
+    auto k = k_sum_points<F, 128>;
+    OG_LAUNCH(ctx, k, 1, 128, 128 * sizeof(XYZZ<F>), d_points, n, d_out, ctx->d_flag);
     return OG_OK;
 }
-#endif  // OG_MSM_G1
-
-#ifdef OG_MSM_G2
-int32_t sum_g2_dev(og_ctx* ctx, const uint8_t* d_points, uint64_t n, uint8_t* d_out128) {
-    auto k = k_sum_points<Fq2, 128>;
-    OG_LAUNCH(ctx, k, 1, 128, 128 * sizeof(G2XYZZ), d_points, n, d_out128, ctx->d_flag);
-    return OG_OK;
-}
-#endif  // OG_MSM_G2
-
 
 // ---- fixed-base window tables ------------------------------------------------------------------------------------
 template <class F>
@@ -1045,20 +789,11 @@ __global__ void __launch_bounds__(64) k_build_table(Affine<F>* __restrict__ tabl
         table[(size_t)w * n + i] = p;
     }
 }
-#ifdef OG_MSM_G1
-int32_t msm_build_table_g1(og_ctx* ctx, G1Affine* d_table, uint32_t n, uint32_t c, uint32_t n_windows) {
-    if (n) OG_LAUNCH(ctx, k_build_table<Fq>, (n + 63) / 64, 64, 0, d_table, n, c, n_windows);
+template <class F>
+int32_t build_table(og_ctx* ctx, Affine<F>* d_table, uint32_t n, uint32_t c, uint32_t n_windows) {
+    if (n) OG_LAUNCH(ctx, k_build_table<F>, (n + 63) / 64, 64, 0, d_table, n, c, n_windows);
     return OG_OK;
 }
-#endif  // OG_MSM_G1
-
-#ifdef OG_MSM_G2
-int32_t msm_build_table_g2(og_ctx* ctx, G2Affine* d_table, uint32_t n, uint32_t c, uint32_t n_windows) {
-    if (n) OG_LAUNCH(ctx, k_build_table<Fq2>, (n + 63) / 64, 64, 0, d_table, n, c, n_windows);
-    return OG_OK;
-}
-#endif  // OG_MSM_G2
-
 
 // ---- fixed-base multiplication by the generators (development setup only) ------------------------------------------
 // gen_table[w * 255 + d - 1] = d * 2^(8w) * G,  w < 32, d in 1..255
@@ -1097,42 +832,48 @@ __global__ void __launch_bounds__(128) k_fixed_mul(const Affine<F>* __restrict__
     out[i] = r;
 }
 
-#ifdef OG_MSM_G2
-static const uint32_t G2_GEN_X0[8] = {0xd992f6edu, 0x46debd5cu, 0xf75edaddu, 0x674322d4u, 0x5e5c4479u, 0x426a0066u, 0x121f1e76u, 0x1800deefu};
-static const uint32_t G2_GEN_X1[8] = {0xaef312c2u, 0x97e485b7u, 0x35a9e712u, 0xf1aa4933u, 0x31fb5d25u, 0x7260bfb7u, 0x920d483au, 0x198e9393u};
-static const uint32_t G2_GEN_Y0[8] = {0x66fa7daau, 0x4ce6cc01u, 0x0c43d37bu, 0xe3d1e769u, 0x8dcb408fu, 0x4aab7180u, 0xdb8c6debu, 0x12c85ea5u};
-static const uint32_t G2_GEN_Y1[8] = {0xd122975bu, 0x55acdadcu, 0x70b38ef3u, 0xbc4b3133u, 0x690c3395u, 0xec9e99adu, 0x585ff075u, 0x090689d0u};
-#endif  // OG_MSM_G2
-
-
-#ifdef OG_MSM_G1
-int32_t fixed_base_mul_g1(og_ctx* ctx, const uint8_t* d_scalars, uint64_t n, G1Affine* d_out) {
-    if (!ctx->g1_fixed) {
-        G1Affine* tab;
-        OG_CUDA(ctx, cudaMalloc(&tab, sizeof(G1Affine) * 32 * 255));
-        G1Affine gen{Fq::from_u32(1), Fq::from_u32(2)};
-        OG_LAUNCH(ctx, k_gen_table<Fq>, 1, 32, 0, gen, tab);
-        ctx->g1_fixed = tab;
+template <class F> struct Generator;
+template <> struct Generator<Fq> {
+    static G1Affine get() { return G1Affine{Fq::from_u32(1), Fq::from_u32(2)}; }
+};
+template <> struct Generator<Fq2> {
+    static G2Affine get() {
+        static const uint32_t X0[8] = {0xd992f6edu, 0x46debd5cu, 0xf75edaddu, 0x674322d4u, 0x5e5c4479u, 0x426a0066u, 0x121f1e76u, 0x1800deefu};
+        static const uint32_t X1[8] = {0xaef312c2u, 0x97e485b7u, 0x35a9e712u, 0xf1aa4933u, 0x31fb5d25u, 0x7260bfb7u, 0x920d483au, 0x198e9393u};
+        static const uint32_t Y0[8] = {0x66fa7daau, 0x4ce6cc01u, 0x0c43d37bu, 0xe3d1e769u, 0x8dcb408fu, 0x4aab7180u, 0xdb8c6debu, 0x12c85ea5u};
+        static const uint32_t Y1[8] = {0xd122975bu, 0x55acdadcu, 0x70b38ef3u, 0xbc4b3133u, 0x690c3395u, 0xec9e99adu, 0x585ff075u, 0x090689d0u};
+        return G2Affine{Fq2{Fq::from_canonical(X0), Fq::from_canonical(X1)}, Fq2{Fq::from_canonical(Y0), Fq::from_canonical(Y1)}};
     }
-    if (n) OG_LAUNCH(ctx, k_fixed_mul<Fq>, (unsigned)((n + 127) / 128), 128, 0, (const G1Affine*)ctx->g1_fixed, d_scalars, n, d_out, ctx->d_flag);
+};
+
+template <class F>
+int32_t fixed_base_mul(og_ctx* ctx, const uint8_t* d_scalars, uint64_t n, Affine<F>* d_out) {
+    void*& fixed = sizeof(F) == 32 ? ctx->g1_fixed : ctx->g2_fixed;    // built on first use, freed with the context
+    if (!fixed) {
+        Affine<F>* tab;
+        OG_CUDA(ctx, cudaMalloc(&tab, sizeof(Affine<F>) * 32 * 255));
+        OG_LAUNCH(ctx, k_gen_table<F>, 1, 32, 0, Generator<F>::get(), tab);
+        fixed = tab;
+    }
+    if (n) OG_LAUNCH(ctx, k_fixed_mul<F>, (unsigned)((n + 127) / 128), 128, 0, (const Affine<F>*)fixed, d_scalars, n, d_out, ctx->d_flag);
     return OG_OK;
 }
-#endif  // OG_MSM_G1
 
-#ifdef OG_MSM_G2
-int32_t fixed_base_mul_g2(og_ctx* ctx, const uint8_t* d_scalars, uint64_t n, G2Affine* d_out) {
-    if (!ctx->g2_fixed) {
-        G2Affine* tab;
-        OG_CUDA(ctx, cudaMalloc(&tab, sizeof(G2Affine) * 32 * 255));
-        G2Affine gen{Fq2{Fq::from_canonical(G2_GEN_X0), Fq::from_canonical(G2_GEN_X1)},
-                     Fq2{Fq::from_canonical(G2_GEN_Y0), Fq::from_canonical(G2_GEN_Y1)}};
-        OG_LAUNCH(ctx, k_gen_table<Fq2>, 1, 32, 0, gen, tab);
-        ctx->g2_fixed = tab;
-    }
-    if (n) OG_LAUNCH(ctx, k_fixed_mul<Fq2>, (unsigned)((n + 127) / 128), 128, 0, (const G2Affine*)ctx->g2_fixed, d_scalars, n, d_out, ctx->d_flag);
-    return OG_OK;
-}
-#endif  // OG_MSM_G2
-
+// ---- the field of this translation unit ---------------------------------------------------------------------------
+#if defined(OG_MSM_G1)
+using MsmField = Fq;
+#elif defined(OG_MSM_G2)
+using MsmField = Fq2;
+#else
+#error "compile msm.cu with -DOG_MSM_G1 or -DOG_MSM_G2"
+#endif
+template int32_t points_to_mont<MsmField>(og_ctx*, const uint8_t*, uint64_t, Affine<MsmField>*);
+template int32_t points_to_bytes<MsmField>(og_ctx*, const Affine<MsmField>*, uint64_t, uint8_t*);
+template int32_t msm_buckets<MsmField>(og_ctx*, const Affine<MsmField>*, const uint32_t*, const uint32_t*, const uint32_t*, uint32_t, uint32_t,
+                                       uint64_t, XYZZ<MsmField>*, XYZZ<MsmField>*, uint32_t*, uint32_t*, XYZZ<MsmField>*, bool);
+template int32_t msm_dev<MsmField>(og_ctx*, const uint8_t*, const uint8_t*, uint64_t, uint8_t*);
+template int32_t sum_points_dev<MsmField>(og_ctx*, const uint8_t*, uint64_t, uint8_t*);
+template int32_t build_table<MsmField>(og_ctx*, Affine<MsmField>*, uint32_t, uint32_t, uint32_t);
+template int32_t fixed_base_mul<MsmField>(og_ctx*, const uint8_t*, uint64_t, Affine<MsmField>*);
 
 }  // namespace og

@@ -24,42 +24,40 @@ struct DigitPlan {
 
 static inline uint32_t msm_windows(uint32_t c) { return (255 + c - 1) / c; }
 
+// The digit sort (msm_sort.cu; the same for both curves).
 // counts[n_keys] must be zero on entry; fills counts, offsets (exclusive scan), sorted entries.
 // Returns total number of entries through *d_total (device pointer inside offsets[n_keys]).
 int32_t msm_sort_digits(og_ctx* ctx, const DigitPlan& plan, uint32_t n_keys, uint32_t* d_counts,
                         uint32_t* d_offsets /* n_keys + 1 */, uint32_t* d_cursor, uint32_t* d_sorted);
 
+// The engine is one set of templates over the coordinate field F: Fq for G1, Fq2 for G2.  msm.cu defines them and is
+// compiled once per field; each of its two objects instantiates every template below for its own field.
+
 // Accumulate every bucket and reduce each group to sum_b (b+1) * bucket_b.
 // d_buckets: n_groups * nb XYZZ scratch; d_lvl: msm_lvl_elems(n_groups, nb) XYZZ scratch;
 // d_heavy: 2 * n_keys + 4 u32 scratch; n_entries_max: upper bound on the sorted entries (sets the heavy-bucket cap);
 // d_perm: n_keys u32 scratch (the sort's cursor array may be reused); result: d_totals[n_groups].
-int32_t msm_buckets_g1(og_ctx* ctx, const G1Affine* d_table, const uint32_t* d_sorted, const uint32_t* d_offsets,
-                       const uint32_t* d_counts, uint32_t n_groups, uint32_t nb, uint64_t n_entries_max, G1XYZZ* d_buckets,
-                       G1XYZZ* d_lvl, uint32_t* d_heavy, uint32_t* d_perm, G1XYZZ* d_totals);
-int32_t msm_buckets_g2(og_ctx* ctx, const G2Affine* d_table, const uint32_t* d_sorted, const uint32_t* d_offsets,
-                       const uint32_t* d_counts, uint32_t n_groups, uint32_t nb, uint64_t n_entries_max, G2XYZZ* d_buckets,
-                       G2XYZZ* d_lvl, uint32_t* d_heavy, uint32_t* d_perm, G2XYZZ* d_totals);
+// few_groups (one-shot MSMs, groups = windows): the levels above the first are reduced as tree sums.
+template <class F>
+int32_t msm_buckets(og_ctx* ctx, const Affine<F>* d_table, const uint32_t* d_sorted, const uint32_t* d_offsets,
+                    const uint32_t* d_counts, uint32_t n_groups, uint32_t nb, uint64_t n_entries_max, XYZZ<F>* d_buckets,
+                    XYZZ<F>* d_lvl, uint32_t* d_heavy, uint32_t* d_perm, XYZZ<F>* d_totals, bool few_groups = false);
 static inline size_t msm_lvl_elems(uint32_t n_groups, uint32_t nb) { return 4 * ((size_t)n_groups * ((nb + 7) / 8) + 16); }   // RED_FAN = 8
 
-// one-shot MSMs on device buffers holding boundary bytes (affine points, canonical scalars)
-int32_t msm_g1_dev(og_ctx* ctx, const uint8_t* d_points, const uint8_t* d_scalars, uint64_t n, uint8_t* d_out64);
-int32_t msm_g2_dev(og_ctx* ctx, const uint8_t* d_points, const uint8_t* d_scalars, uint64_t n, uint8_t* d_out128);
-int32_t sum_g1_dev(og_ctx* ctx, const uint8_t* d_points, uint64_t n, uint8_t* d_out64);
-int32_t sum_g2_dev(og_ctx* ctx, const uint8_t* d_points, uint64_t n, uint8_t* d_out128);
+// one-shot MSM on device buffers holding boundary bytes (affine points, canonical scalars); d_out: one point
+template <class F> int32_t msm_dev(og_ctx* ctx, const uint8_t* d_points, const uint8_t* d_scalars, uint64_t n, uint8_t* d_out);
+// plain sum of n points in boundary bytes
+template <class F> int32_t sum_points_dev(og_ctx* ctx, const uint8_t* d_points, uint64_t n, uint8_t* d_out);
 
 // boundary conversions for points
-int32_t g1_bytes_to_mont(og_ctx* ctx, const uint8_t* d_in, uint64_t n, G1Affine* d_out);
-int32_t g2_bytes_to_mont(og_ctx* ctx, const uint8_t* d_in, uint64_t n, G2Affine* d_out);
-int32_t g1_mont_to_bytes(og_ctx* ctx, const G1Affine* d_in, uint64_t n, uint8_t* d_out);
-int32_t g2_mont_to_bytes(og_ctx* ctx, const G2Affine* d_in, uint64_t n, uint8_t* d_out);
+template <class F> int32_t points_to_mont(og_ctx* ctx, const uint8_t* d_in, uint64_t n, Affine<F>* d_out);
+template <class F> int32_t points_to_bytes(og_ctx* ctx, const Affine<F>* d_in, uint64_t n, uint8_t* d_out);
 
 // fixed-base window tables: table[w * n + i] = 2^(c*w) * P_i  (w < n_windows), affine Montgomery.
 // table[0..n) must already hold the points.
-int32_t msm_build_table_g1(og_ctx* ctx, G1Affine* d_table, uint32_t n, uint32_t c, uint32_t n_windows);
-int32_t msm_build_table_g2(og_ctx* ctx, G2Affine* d_table, uint32_t n, uint32_t c, uint32_t n_windows);
+template <class F> int32_t build_table(og_ctx* ctx, Affine<F>* d_table, uint32_t n, uint32_t c, uint32_t n_windows);
 
-// out[i] = scalars[i] * generator (setup): scalars canonical bytes on device, out affine Montgomery
-int32_t fixed_base_mul_g1(og_ctx* ctx, const uint8_t* d_scalars, uint64_t n, G1Affine* d_out);
-int32_t fixed_base_mul_g2(og_ctx* ctx, const uint8_t* d_scalars, uint64_t n, G2Affine* d_out);
+// out[i] = scalars[i] * generator of G1 / G2 (setup): scalars canonical bytes on device, out affine Montgomery
+template <class F> int32_t fixed_base_mul(og_ctx* ctx, const uint8_t* d_scalars, uint64_t n, Affine<F>* d_out);
 
 }  // namespace og

@@ -2,7 +2,7 @@
 // the clear": tau, alpha, beta, gamma, delta are inputs, so that every pk/vk byte is reproducible and
 // can be compared with oracle/groth16.py).  A production deployment would load a ceremony's key with
 // og_load_pk instead.  QAP evaluation at tau is ~10^5 host field operations; the ~1.6*10^5
-// fixed-base scalar multiplications run on the GPU (msm.cu: fixed_base_mul_*).
+// fixed-base scalar multiplications run on the GPU (msm.cu: fixed_base_mul).
 // Conventions: DESIGN.md section 4 (domain, input-consistency rows, coset-Lagrange H query).
 #include "groth16.cuh"
 #include "msm.cuh"
@@ -58,6 +58,19 @@ static void put_csr(std::vector<uint8_t>& v, const Csr& M) {
     put_bytes(v, reinterpret_cast<const uint8_t*>(M.row_ptr.data()), 4 * M.row_ptr.size());
     put_bytes(v, reinterpret_cast<const uint8_t*>(M.col.data()), 4 * M.col.size());
     for (const Fr& c : M.val) { uint8_t b[32]; host_store(b, c); put_bytes(v, b, 32); }
+}
+
+// out = boundary bytes of scalars[i] * generator (G1 or G2) for the n canonical scalars in s, through the setup's scratch slots
+template <class F>
+static int32_t generator_mul(og_ctx* ctx, const std::vector<uint8_t>& s, uint64_t n, uint8_t* d_s, uint8_t* d_pts, uint8_t* d_bytes,
+                             std::vector<uint8_t>& out) {
+    out.resize(sizeof(Affine<F>) * n);
+    OG_CUDA(ctx, cudaMemcpyAsync(d_s, s.data(), 32 * n, cudaMemcpyHostToDevice, ctx->stream));
+    OG_TRY(fixed_base_mul<F>(ctx, d_s, n, reinterpret_cast<Affine<F>*>(d_pts)));
+    OG_TRY(points_to_bytes(ctx, reinterpret_cast<Affine<F>*>(d_pts), n, d_bytes));
+    OG_CUDA(ctx, cudaMemcpyAsync(out.data(), d_bytes, out.size(), cudaMemcpyDeviceToHost, ctx->stream));
+    OG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return OG_OK;
 }
 
 int32_t setup_withdraw(og_ctx* ctx, uint32_t depth, const uint8_t* toxic160, uint8_t* pk_out, uint64_t* pk_len,
@@ -116,16 +129,9 @@ int32_t setup_withdraw(og_ctx* ctx, uint32_t depth, const uint8_t* toxic160, uin
     OG_SLOT(ctx, d_s, uint8_t, S_SETUP_A, 32 * (n1 > n2 ? n1 : n2));
     OG_SLOT(ctx, d_pts, uint8_t, S_SETUP_B, sizeof(G2Affine) * (n1 > n2 ? n1 : n2));
     OG_SLOT(ctx, d_bytes, uint8_t, S_SETUP_C, 128 * (n1 > n2 ? n1 : n2));
-    std::vector<uint8_t> p1(64 * n1), p2(128 * n2);
-    OG_CUDA(ctx, cudaMemcpyAsync(d_s, s1.data(), 32 * n1, cudaMemcpyHostToDevice, ctx->stream));
-    OG_TRY(fixed_base_mul_g1(ctx, d_s, n1, reinterpret_cast<G1Affine*>(d_pts)));
-    OG_TRY(g1_mont_to_bytes(ctx, reinterpret_cast<G1Affine*>(d_pts), n1, d_bytes));
-    OG_CUDA(ctx, cudaMemcpyAsync(p1.data(), d_bytes, 64 * n1, cudaMemcpyDeviceToHost, ctx->stream));
-    OG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    OG_CUDA(ctx, cudaMemcpyAsync(d_s, s2.data(), 32 * n2, cudaMemcpyHostToDevice, ctx->stream));
-    OG_TRY(fixed_base_mul_g2(ctx, d_s, n2, reinterpret_cast<G2Affine*>(d_pts)));
-    OG_TRY(g2_mont_to_bytes(ctx, reinterpret_cast<G2Affine*>(d_pts), n2, d_bytes));
-    OG_CUDA(ctx, cudaMemcpyAsync(p2.data(), d_bytes, 128 * n2, cudaMemcpyDeviceToHost, ctx->stream));
+    std::vector<uint8_t> p1, p2;
+    OG_TRY(generator_mul<Fq>(ctx, s1, n1, d_s, d_pts, d_bytes, p1));
+    OG_TRY(generator_mul<Fq2>(ctx, s2, n2, d_s, d_pts, d_bytes, p2));
     OG_TRY(check_flag(ctx));
 
     const uint8_t* alpha1 = p1.data(); const uint8_t* beta1 = p1.data() + 64; const uint8_t* delta1 = p1.data() + 128;

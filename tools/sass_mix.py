@@ -10,7 +10,7 @@ import re
 import subprocess
 import sys
 
-HOT = ["k_bucket_acc_sm1", "k_bucket_acc_sm", "k_reduce_level", "k_ntt_pass2", "k_digits", "k_digits_count_tiled", "k_merkle_paths",
+HOT = ["k_bucket_acc", "k_reduce_level", "k_ntt_pass2", "k_digits", "k_digits_count_tiled", "k_merkle_paths",
        "k_withdraw_witness", "k_abc", "k_pointwise", "k_bucket_heavy", "k_assemble_g1", "k_tree_append_level", "k_horner", "k_bjj"]
 COLS = ["IMAD.WIDE", "IMAD other", "IADD3", "LOP3/SHF/SEL", "LDL", "STL", "LDS", "STS", "LDG", "STG", "ATOM/RED", "SHFL", "BAR", "CALL", "total"]
 BLACKWELL = ("UTMALDG", "UTMASTG", "UBLKCP", "UTCHMMA", "UTCIMMA", "UTCQMMA", "UTCOMMA", "UTCBAR", "LDTM", "STTM", "SYNCS", "UTMAPF", "HGMMA", "TCGEN")
